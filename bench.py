@@ -2,7 +2,7 @@
 """Benchmark of the BAE+CAA enhancement hot path (BASELINE.json: 720p enhanced frames/s + roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2|C3|C4|C5] [--frames T] [--clips n]
-                    [--impl ours|reference]
+                    [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one batch of synthetic clips of the selected BASELINE.json config per GPU through the registry-built
 generator: C2 (default at N=1) one REDS4-shape clip 1280x720x100, per-frame random QPs, CRF cycling 15/25/35 over the
@@ -293,6 +293,31 @@ def _emit(line):
     out.flush()
 
 
+#: --dump-outputs keeps at most this many values of the enhanced frames (16 MB of float32)
+DUMP_MAX_VALUES = 1 << 22
+
+
+def dump_outputs(path, out):
+    """--dump-outputs: what the last timed step returned to its caller, as .npy files under `path`.
+
+    frames.npy         the enhanced frames (n, T, 3, H, W) float32, when they hold at most DUMP_MAX_VALUES values
+    frames_sample.npy  otherwise: the values at DUMP_MAX_VALUES flat positions drawn with a fixed seed, in ascending
+                       position order (the same positions for the same arguments)
+    frame_metrics.npy  (n, T, 2) float32 per-frame max-abs and mean square of the whole frames (driver.frame_metrics)
+    """
+    import numpy as np
+    from pnpvcve_b200 import driver
+    os.makedirs(path, exist_ok=True)
+    flat = out.reshape(-1)
+    if flat.numel() <= DUMP_MAX_VALUES:
+        np.save(os.path.join(path, "frames.npy"), out.float().cpu().numpy())
+    else:
+        g = torch.Generator().manual_seed(0)
+        pos = torch.randint(flat.numel(), (DUMP_MAX_VALUES,), generator=g).sort().values
+        np.save(os.path.join(path, "frames_sample.npy"), flat[pos.to(flat.device)].float().cpu().numpy())
+    np.save(os.path.join(path, "frame_metrics.npy"), driver.frame_metrics(out).cpu().numpy())
+
+
 def timed_resident(net, batches, steps, warmup, dev):
     """frames/s of `steps` resident steps (CUDA events, no events inside the steps)."""
     from pnpvcve_b200 import synthetic
@@ -349,7 +374,9 @@ def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps of the headline value and of the e2e, e2e_sideinfo (three repetitions) and "
+                         "frame_windows blocks; other_configs and the kernel profiling pass use fixed counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", default=None, choices=sorted(CONFIGS),
                     help="BASELINE.json config (default: C2 at --gpus 1, C3 at --gpus > 1)")
@@ -362,7 +389,13 @@ def main():
     ap.add_argument("--no-windows", action="store_true", help="skip the frame-window (single clip, strong scaling) block")
     ap.add_argument("--prof-every", type=int, default=8,
                     help="bracket every N-th launch of the profiled kernels with CUDA events")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frames the last timed step computed (rank 0) as .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the CUDA path's frames; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -417,10 +450,15 @@ def main():
         launches = 0
         e0.record()
         for i in range(args.steps):
-            step_resident(args.warmup + i)
+            out = step_resident(args.warmup + i)
             launches += net.gpu_launches
+            if i + 1 < args.steps:
+                del out                            # only the last step's frames outlive their step
         e1.record()
         barrier()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, out)
+        del out
         # Per-kernel durations come from a SEPARATE pass of the same steps, right behind the timed one (same
         # clocks, same thermal state): an event record between two launches defeats programmatic dependent
         # launch for both neighbours, and bracketing every 8th launch was measured to slow the whole step by
@@ -581,7 +619,7 @@ def main():
                 driver.enhance_windows(net, [wclip], wlen, rank, world, gather_output=True)
             barrier()
             g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            wsteps = max(2, args.steps)
+            wsteps = args.steps
             g0.record()
             for _ in range(wsteps):
                 driver.enhance_windows(net, [wclip], wlen, rank, world, gather_output=True)

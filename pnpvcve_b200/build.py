@@ -19,10 +19,10 @@ def _newest_source_mtime():
     return m
 
 
-def build(force=False, verbose=False):
-    """Compile when the library is missing or older than its sources.  Returns the .so path."""
-    if not force and os.path.isfile(LIB) and os.path.getmtime(LIB) >= _newest_source_mtime():
-        return LIB
+def build(force=False, verbose=False, lib=LIB):
+    """Compile `lib` (default: the in-tree library) when it is missing or older than its sources.  Returns its path."""
+    if not force and os.path.isfile(lib) and os.path.getmtime(lib) >= _newest_source_mtime():
+        return lib
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
     flags = list(NVCC_FLAGS)
     if os.environ.get("PNP_DIAG", "0") != "0":     # diagnostics build for tools/ (what-if bits, clock traces)
@@ -33,13 +33,13 @@ def build(force=False, verbose=False):
         flags.append("-DPNP_STEP_RING_LOG2=" + os.environ["PNP_STEP_RING_LOG2"])
     if os.environ.get("PNP_SPIN_LIMIT"):           # stress runs: trap a stuck pipeline after fewer polls
         flags.append("-DPNP_SPIN_LIMIT=" + os.environ["PNP_SPIN_LIMIT"])
-    cmd = [nvcc] + flags + ["-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES]
+    cmd = [nvcc] + flags + ["-o", lib] + [os.path.join(CSRC, s) for s in SOURCES]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or res.returncode != 0:
         sys.stderr.write(res.stdout + res.stderr)
     if res.returncode != 0:
-        raise RuntimeError("nvcc failed building libpnpvcve.so")
-    return LIB
+        raise RuntimeError(f"nvcc failed building {lib}")
+    return lib
 
 
 if __name__ == "__main__":

@@ -297,6 +297,11 @@ conv3x3_rows_kernel(const __grid_constant__ ConvParams p) {
   auto ewait = [&](uint32_t bar, uint32_t parity, int tag) {      // whole (converged) warp
     if (hot_waits) mbar_wait(bar, parity, tag); else mbar_wait_warp(bar, parity, tag, hint_ns);
   };
+  // debug bit 2048: every output row of the epilogue starts ~2 us late, so the epilogue trails the MMA issuer by a full
+  // accumulator ring -- the schedule the step-barrier ring (kStepRing) must survive; results stay exact
+  auto slow_epilogue = [&]() {
+    if (PNP_DBG(2048)) __nanosleep(2000);
+  };
   const uint32_t w_smem = sbase + L.w;
   const uint32_t a_smem = sbase + L.a;
   const uint32_t aux_smem = sbase + L.aux;
@@ -839,6 +844,7 @@ conv3x3_rows_kernel(const __grid_constant__ ConvParams p) {
           }
           const bool trm = PNP_TRACING && blockIdx.x == 0 && ord < 64 && warp == 2 && lane == 0;
           if (trm) p.trace[2816 + ord * 4 + 0] = clock64();
+          slow_epilogue();
           mbar_wait(smem_u32(&misc->step_done[sc_last & (kStepRing - 1)]), (sc_last >> kStepShift) & 1, 9);
           if (trm) p.trace[2816 + ord * 4 + 1] = clock64();
           tc_fence_after();
@@ -993,6 +999,7 @@ conv3x3_rows_kernel(const __grid_constant__ ConvParams p) {
 
     Ring ior(n_io);
     while (cur.valid) {
+      slow_epilogue();
       const Segment& s = cur.s;
       const int o = cur.o;
       const uint32_t ord = cur.ord;

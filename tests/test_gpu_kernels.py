@@ -498,24 +498,29 @@ def test_fetch_pinned_copies_without_the_copy_engine(dev):
     assert lib.pnp_fetch_pinned(dst.data_ptr(), pageable.data_ptr(), 64, None) != 0
 
 
-def test_conv_720p_survives_a_slow_epilogue(dev):
+def test_conv_720p_survives_a_slow_epilogue(dev, tmp_path, monkeypatch):
     """Regression for the step-barrier ABA (pnp_conv_rows.cu, kStepRing): with 8 step barriers the CTA whose tile range
     ends a few rows into a new column (720p: CTA 102) dead-locked whenever its epilogue fell a full accumulator ring
-    behind the MMA thread -- once in ~10^6 launches natively, every time under compute-sanitizer, which slows the
-    epilogue warps but not the tensor pipe.  Runs the 720p conv variants (both kernel forms) under memcheck: must pass,
-    with no memory errors."""
-    import shutil
+    behind the MMA thread -- once in ~10^6 launches natively, every time the epilogue warps are slowed but the tensor
+    pipe is not.  A diagnostics build of the library (PNP_DIAG, debug bit 2048) delays every epilogue row by ~2 us;
+    the 720p conv variants (both kernel forms) must run through with it and stay bit-identical.  That delay does reach
+    the full-ring schedule (tools/epilogue_lag.py, profiles/r03_epilogue_lag.log; CTA 0 of a 720p launch, B200 at
+    1000 W): when the epilogue takes a row, the issuer has begun 5 steps beyond the one completing it (plain conv; 2 with
+    the partition 1x1 convs), i.e. all 8 (5) accumulators are held, against 1 step without the delay."""
     import subprocess
     import sys
-    tool = shutil.which("compute-sanitizer") or "/usr/local/cuda/bin/compute-sanitizer"
-    if not os.path.exists(tool):
-        pytest.skip("compute-sanitizer not installed")
-    cmd = [tool, "--tool", "memcheck", "--error-exitcode", "9", sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu",
-           "-x", "-q", "-k", "pair_form and 720"]
-    res = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    from pnpvcve_b200 import build
+    lib = str(tmp_path / "libpnpvcve_diag.so")
+    monkeypatch.setenv("PNP_DIAG", "1")
+    build.build(force=True, lib=lib)
+    env = dict(os.environ, PNP_LIB_PATH=lib, PNP_DEBUG_SKIP="2048")
+    cmd = [sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-x", "-q", "-p", "no:cacheprovider",
+           "-k", "pair_form and 720"]
+    res = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=env,
+                         cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     tail = (res.stdout + res.stderr)[-1500:]
     assert res.returncode == 0, tail
-    assert "1 passed" in res.stdout and "ERROR SUMMARY: 0 errors" in res.stdout + res.stderr, tail
+    assert "1 passed" in res.stdout, tail
 
 
 def test_table_mode_launches_equal_static_launches(dev):

@@ -127,7 +127,9 @@ def test_config_loader_base_inheritance(tmp_path):
     assert dict(cfg.data.test) == {"type": "B"}
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not refshim.available(),
+                    reason="reads the upstream PnP-VCVE config files from its source tree (PNP_REFERENCE_ROOT), which is "
+                           "not part of this repository")
 @pytest.mark.parametrize("cfgname", ["HR_davis_LR_128x128.py", "HR_davis_LR_128x128_IPB.py",
                                      "HR_davis_LR_128x128_IPB_LR_test.py"])
 def test_reference_configs_build_unchanged(cfgname):

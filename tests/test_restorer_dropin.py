@@ -12,7 +12,10 @@ from oracle import refshim
 import pnpvcve_b200 as P
 from pnpvcve_b200 import synthetic, weights
 
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(
+    not refshim.available(),
+    reason="executes the upstream PnP-VCVE restorer code from its source tree (PNP_REFERENCE_ROOT), which is not part of "
+           "this repository")
 
 GENERATOR_CFG = dict(
     type="IconVSR_restore_wo_refill_mv_ipb_fast_domain_dynamic_with_par",
