@@ -197,6 +197,25 @@ int pnp_mv_rasterize(const float* records, const int32_t* frame_offsets, const i
 int pnp_frame_quality(const float* a, int64_t a_sf, int64_t a_sc, int64_t a_sy, const float* b, int64_t b_sf,
                       int64_t b_sc, int64_t b_sy, int F, int H, int W, int crop_border, unsigned long long* sse,
                       double* ssim_sum, void* stream);
+/* The same metrics with each operand fp32 or uint8: *_is_u8 = 1 makes that operand a uint8 (F,3,H,W) view (strides in
+ * bytes) whose values are taken as they are; fp32 operands are quantised as above, so every operand mix sees the same
+ * uint8 values: sse is identical, and so is every per-block float64 partial of ssim_sum (the partials meet in float64
+ * atomics, whose order -- and with it the last bits of the total -- varies between launches for any operand types).
+ * pnp_frame_quality is the fp32 / fp32 case. */
+int pnp_frame_quality_u8(const void* a, int a_is_u8, int64_t a_sf, int64_t a_sc, int64_t a_sy, const void* b,
+                         int b_is_u8, int64_t b_sf, int64_t b_sc, int64_t b_sy, int F, int H, int W, int crop_border,
+                         unsigned long long* sse, double* ssim_sum, void* stream);
+
+/*
+ * 8-bit frames -> fp32 lq.  The reference's loader decodes PNGs to uint8 and RescaleToZeroOne computes
+ * img.astype(np.float32) / 255. (mmedit/datasets/pipelines/normalization.py:93-99); dst = the correctly rounded fp32
+ * quotient v / 255 of every sample (not v * (1/255f), which differs for 126 of the 256 values).
+ *   src : uint8 (F,3,H,W) view, unit x stride; s_sf/s_sc/s_sy = frame / channel / row strides in bytes
+ *   dst : fp32 (F,3,H,W) view, unit x stride; d_sf/d_sc/d_sy in elements
+ * F <= 65535, H <= 21845.
+ */
+int pnp_unit_from_u8(const uint8_t* src, int64_t s_sf, int64_t s_sc, int64_t s_sy, float* dst, int64_t d_sf,
+                     int64_t d_sc, int64_t d_sy, int F, int H, int W, void* stream);
 
 /*
  * K2/K3/K5 -- fused 3x3 convolution on tcgen05 tensor cores (implicit GEMM, TMA fed, TMEM
@@ -205,7 +224,7 @@ int pnp_frame_quality(const float* a, int64_t a_sf, int64_t a_sc, int64_t a_sy, 
  *   acc  = conv3x3(src, W) [+ conv1x1(aux, Waux)]
  *   v    = acc * scale + bias [+ sum_k par_k * conv1x1_k(src)] [+ idt]      (fp32)
  *   out  = act(v)                       -> bf16 NHWC               (mode PNP_CONV_BF16)
- *   outf = v[0:3] + lq (or up4(lq))     -> fp32 NCHW view          (mode PNP_CONV_LAST)
+ *   outf = v[0:3] + lq (or up4(lq))     -> fp32 NCHW view          (mode PNP_CONV_LAST; uint8 with out_u8)
  * Reference call sites: ResidualBlockNoBNDynamic_drt.forward (sr_backbone_utils.py:304-333),
  * input_conv (basicvsr_net.py:484,515), conv_hr/conv_last (iconvsr_ipb_par.py:144-146).
  */
@@ -226,7 +245,7 @@ typedef struct pnp_conv_desc {
   int64_t par_sn, par_sc, par_sy;
   const float* lq;     /* PNP_CONV_LAST: fp32 (N,3,H,W) view */
   int64_t lq_sn, lq_sc, lq_sy;
-  float* outf;         /* PNP_CONV_LAST: fp32 (N,3,H,W) view */
+  float* outf;         /* PNP_CONV_LAST: fp32 (N,3,H,W) view (uint8 with out_u8) */
   int64_t of_sn, of_sc, of_sy;
   int32_t N, H, W;
   int32_t tap_n;       /* 64, or 16 for PNP_CONV_LAST */
@@ -263,7 +282,11 @@ typedef struct pnp_conv_desc {
   int32_t src_images, aux_images, idt_images, out_images;
   int32_t aux_channels; /* channels per pixel of `aux`: 64 (or 0) = a (N,H,W,64) tensor; 32 = a (N,H,W,32) tensor of 64-byte
                           pixels as pnp_lr_im2col writes it with dst_channels = 32 (aux_k16 <= 2) */
-  int32_t reserved0;
+  int32_t out_u8;      /* PNP_CONV_LAST: 1 = `outf` is a uint8 (N,3,H,W) view (of_* strides in bytes) and receives tensor2img's
+                          value of every output sample (mmedit/core/misc.py:9-74): the same fp32 v + bias + lq as the fp32
+                          store, clamped to [0,1], x255 (fp32), rounded half to even -- the uint8 frame the reference scores or
+                          writes, and what pnp_frame_quality computes from the fp32 frame.  0 = fp32 store (the only value
+                          accepted for PNP_CONV_BF16). */
 } pnp_conv_desc;
 
 int pnp_conv3x3(const pnp_conv_desc* desc, void* stream);

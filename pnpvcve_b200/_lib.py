@@ -20,7 +20,8 @@ EXPORTS = [
     "pnp_graph_begin", "pnp_graph_end", "pnp_graph_launch", "pnp_graph_destroy", "pnp_set_step", "pnp_fetch_pinned",
     "pnp_mv_warp", "pnp_mv_warp_dyn", "pnp_lr_im2col", "pnp_lr_im2col_dyn", "pnp_pack_conv3x3_rowstack",
     "pnp_pack_rows", "pnp_pack_aux", "pnp_pack_mix_blocks",
-    "pnp_caa_heads", "pnp_mix_bias", "pnp_mv_rasterize", "pnp_conv3x3", "pnp_frame_quality",
+    "pnp_caa_heads", "pnp_mix_bias", "pnp_mv_rasterize", "pnp_conv3x3", "pnp_frame_quality", "pnp_frame_quality_u8",
+    "pnp_unit_from_u8",
 ]
 
 _c = ctypes
@@ -48,7 +49,7 @@ class ConvDesc(_c.Structure):
         ("img_off", _vp),
         ("dyn", DynRef),
         ("src_images", _c.c_int32), ("aux_images", _c.c_int32), ("idt_images", _c.c_int32), ("out_images", _c.c_int32),
-        ("aux_channels", _c.c_int32), ("reserved0", _c.c_int32),
+        ("aux_channels", _c.c_int32), ("out_u8", _c.c_int32),
     ]
 
 
@@ -81,6 +82,8 @@ _PROTOS = {
     "pnp_mv_rasterize": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pnp_conv3x3": (_i, [_c.POINTER(ConvDesc), _vp]),
     "pnp_frame_quality": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "pnp_frame_quality_u8": (_i, [_vp, _i, _i64, _i64, _i64, _vp, _i, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "pnp_unit_from_u8": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _vp]),
 }
 
 _lib = None

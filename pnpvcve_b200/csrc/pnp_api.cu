@@ -180,13 +180,38 @@ int make_map(CUtensorMap* m, const void* base, int N, int H, int W, int box_w, l
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// pnp_frame_quality / pnp_frame_quality_u8: one implementation, operands fp32 or uint8
+int frame_quality(const char* name, const void* a, bool a_u8, int64_t a_sf, int64_t a_sc, int64_t a_sy, const void* b,
+                  bool b_u8, int64_t b_sf, int64_t b_sc, int64_t b_sy, int F, int H, int W, int crop_border,
+                  unsigned long long* sse, double* ssim_sum, void* stream) {
+  if (!a || !b || !sse || !ssim_sum) return fail(PNP_ERR_ARG, "%s: null pointer", name);
+  if (F < 1 || crop_border < 0 || H - 2 * crop_border < 11 || W - 2 * crop_border < 11)
+    return fail(PNP_ERR_ARG, "%s: the cropped frame must be at least 11 x 11", name);
+  if ((long long)F * 3 > 65535) return fail(PNP_ERR_ARG, "%s: at most 21845 frames per call", name);
+  DeviceInfo* d;
+  int rc = device_info(&d);
+  if (rc) return rc;
+  // cv2.getGaussianKernel(11, 1.5): exp(-(i-5)^2 / (2 sigma^2)), normalised to sum 1 (float64)
+  double g[11], s = 0.0;
+  for (int i = 0; i < 11; ++i) {
+    g[i] = exp(-((double)(i - 5) * (i - 5)) / (2.0 * 1.5 * 1.5));
+    s += g[i];
+  }
+  for (int i = 0; i < 11; ++i) g[i] /= s;
+  const int ch_first = crop_border != 0 ? 2 : 0, n_ch = crop_border != 0 ? 1 : 3;
+  cudaError_t e = pnp::launch_frame_quality(a, a_u8, a_sf, a_sc, a_sy, b, b_u8, b_sf, b_sc, b_sy, F, H, W, crop_border,
+                                            ch_first, n_ch, g, sse, ssim_sum, d->sms, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? PNP_OK : cuda_fail(e, name);
+}
+
 }  // namespace
 
 extern "C" {
 
 static_assert(sizeof(pnp_conv_desc) == 280 && offsetof(pnp_conv_desc, out_spx) == 184 &&
                   offsetof(pnp_conv_desc, img_off) == 224 && offsetof(pnp_conv_desc, dyn) == 232 &&
-                  offsetof(pnp_conv_desc, src_images) == 256 && offsetof(pnp_conv_desc, aux_channels) == 272,
+                  offsetof(pnp_conv_desc, src_images) == 256 && offsetof(pnp_conv_desc, aux_channels) == 272 &&
+                  offsetof(pnp_conv_desc, out_u8) == 276,
               "pnp_conv_desc layout is part of the ABI (mirrored by pnpvcve_b200/_lib.py: ConvDesc)");
 int pnp_abi_version(void) { return 10; }
 
@@ -439,24 +464,28 @@ int pnp_mv_rasterize(const float* records, const int32_t* frame_offsets, const i
 int pnp_frame_quality(const float* a, int64_t a_sf, int64_t a_sc, int64_t a_sy, const float* b, int64_t b_sf,
                       int64_t b_sc, int64_t b_sy, int F, int H, int W, int crop_border, unsigned long long* sse,
                       double* ssim_sum, void* stream) {
-  if (!a || !b || !sse || !ssim_sum) return fail(PNP_ERR_ARG, "pnp_frame_quality: null pointer");
-  if (F < 1 || crop_border < 0 || H - 2 * crop_border < 11 || W - 2 * crop_border < 11)
-    return fail(PNP_ERR_ARG, "pnp_frame_quality: the cropped frame must be at least 11 x 11");
-  if ((long long)F * 3 > 65535) return fail(PNP_ERR_ARG, "pnp_frame_quality: at most 21845 frames per call");
+  return frame_quality("pnp_frame_quality", a, false, a_sf, a_sc, a_sy, b, false, b_sf, b_sc, b_sy, F, H, W, crop_border,
+                       sse, ssim_sum, stream);
+}
+
+int pnp_frame_quality_u8(const void* a, int a_is_u8, int64_t a_sf, int64_t a_sc, int64_t a_sy, const void* b,
+                         int b_is_u8, int64_t b_sf, int64_t b_sc, int64_t b_sy, int F, int H, int W, int crop_border,
+                         unsigned long long* sse, double* ssim_sum, void* stream) {
+  return frame_quality("pnp_frame_quality_u8", a, a_is_u8 != 0, a_sf, a_sc, a_sy, b, b_is_u8 != 0, b_sf, b_sc, b_sy, F,
+                       H, W, crop_border, sse, ssim_sum, stream);
+}
+
+int pnp_unit_from_u8(const uint8_t* src, int64_t s_sf, int64_t s_sc, int64_t s_sy, float* dst, int64_t d_sf,
+                     int64_t d_sc, int64_t d_sy, int F, int H, int W, void* stream) {
+  if (!src || !dst) return fail(PNP_ERR_ARG, "pnp_unit_from_u8: null pointer");
+  if (F < 1 || F > 65535 || H < 1 || H > 21845 || W < 1)
+    return fail(PNP_ERR_ARG, "pnp_unit_from_u8: bad shape (1 <= F <= 65535, 1 <= H <= 21845)");
   DeviceInfo* d;
   int rc = device_info(&d);
   if (rc) return rc;
-  // cv2.getGaussianKernel(11, 1.5): exp(-(i-5)^2 / (2 sigma^2)), normalised to sum 1 (float64)
-  double g[11], s = 0.0;
-  for (int i = 0; i < 11; ++i) {
-    g[i] = exp(-((double)(i - 5) * (i - 5)) / (2.0 * 1.5 * 1.5));
-    s += g[i];
-  }
-  for (int i = 0; i < 11; ++i) g[i] /= s;
-  const int ch_first = crop_border != 0 ? 2 : 0, n_ch = crop_border != 0 ? 1 : 3;
-  cudaError_t e = pnp::launch_frame_quality(a, a_sf, a_sc, a_sy, b, b_sf, b_sc, b_sy, F, H, W, crop_border, ch_first,
-                                            n_ch, g, sse, ssim_sum, d->sms, static_cast<cudaStream_t>(stream));
-  return e == cudaSuccess ? PNP_OK : cuda_fail(e, "pnp_frame_quality");
+  cudaError_t e = pnp::launch_unit_from_u8(src, s_sf, s_sc, s_sy, dst, d_sf, d_sc, d_sy, F, H, W,
+                                           static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? PNP_OK : cuda_fail(e, "pnp_unit_from_u8");
 }
 
 int pnp_conv3x3(const pnp_conv_desc* c, void* stream) {
@@ -489,6 +518,7 @@ int pnp_conv3x3(const pnp_conv_desc* c, void* stream) {
   if (strided_out && (last || c->out_spx < 64 || c->out_sy < c->out_spx * c->W || (c->N > 1 && c->out_sn < c->out_sy * c->H) ||
                       ((c->out_spx | c->out_sy | c->out_sn) & 7)))
     return fail(PNP_ERR_ARG, "pnp_conv3x3: out strides must be non-overlapping multiples of 8 elements (PNP_CONV_BF16 only)");
+  if (c->out_u8 && !last) return fail(PNP_ERR_ARG, "pnp_conv3x3: out_u8 needs PNP_CONV_LAST");
   if (c->lq_up4 && (!last || (c->H & 3) || (c->W & 3)))
     return fail(PNP_ERR_ARG, "pnp_conv3x3: lq_up4 needs PNP_CONV_LAST and H, W multiples of 4");
   if (!aligned16(c->src) || (c->wpack && !aligned16(c->wpack)) || (c->aux && !aligned16(c->aux)) ||
@@ -528,6 +558,7 @@ int pnp_conv3x3(const pnp_conv_desc* c, void* stream) {
   p.lq_sn = c->lq_sn; p.lq_sc = c->lq_sc; p.lq_sy = c->lq_sy;
   p.outf = c->outf;
   p.of_sn = c->of_sn; p.of_sc = c->of_sc; p.of_sy = c->of_sy;
+  p.out_u8 = c->out_u8 ? 1 : 0;
   p.H = c->H; p.W = c->W; p.N = c->N;
   p.strips = (c->W + pnp::kTilePx - 1) / pnp::kTilePx;
   const long long tiles = (long long)c->N * p.strips * c->H;

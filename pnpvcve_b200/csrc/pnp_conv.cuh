@@ -54,7 +54,7 @@ struct ConvParams {
   long long par_sn, par_sc, par_sy;
   const float* lq;      // kModeLast: (n,3,H,W) fp32 view added to the output
   long long lq_sn, lq_sc, lq_sy;
-  float* outf;          // kModeLast: (n,3,H,W) fp32 view
+  float* outf;          // kModeLast: (n,3,H,W) fp32 view -- uint8 with out_u8 (strides then in bytes)
   long long of_sn, of_sc, of_sy;
   int H, W, N, strips;
   int tiles_total, tiles_per_cta;
@@ -81,6 +81,7 @@ struct ConvParams {
   int n_io;             // id/out staging slots
   long long* trace;     // PNP_DIAG builds: device buffer for per-tile clock64 stamps of CTA 0
   int debug_skip;       // PNP_DIAG builds: what-if profiling bits (results are WRONG)
+  int out_u8;           // kModeLast: store tensor2img's uint8 value of each output sample (quant_u8) instead of fp32
 };
 
 // sparse_val eval path of the reference (sr_backbone_utils.py:294-302, basicvsr_net.py:511-514): per class the

@@ -28,6 +28,7 @@
 #include <type_traits>
 
 #include "pnp_conv.cuh"
+#include "pnp_ops.cuh"
 #include "pnp_ptx.cuh"
 
 // Diagnostics (what-if bits, clock traces) exist only in PNP_DIAG builds (PNP_DIAG=1 python -m pnpvcve_b200.build):
@@ -1034,10 +1035,21 @@ conv3x3_rows_kernel(const __grid_constant__ ConvParams p) {
         tc_fence_before();
         acc_release(slot);
         if (valid && half == 0) {
-          float* op = outf_g + (long long)s.n * p.of_sn + (long long)y * p.of_sy + x;
-          op[0] = v[0] + misc->bias[0] + r0;
-          op[p.of_sc] = v[1] + misc->bias[1] + r1;
-          op[2 * p.of_sc] = v[2] + misc->bias[2] + r2;
+          const long long o_off = (long long)s.n * p.of_sn + (long long)y * p.of_sy + x;
+          const float o0 = v[0] + misc->bias[0] + r0, o1 = v[1] + misc->bias[1] + r1, o2 = v[2] + misc->bias[2] + r2;
+          // the same fp32 sums, stored as tensor2img's uint8 values (kModeLast never has a partition operand: the kPar
+          // instances leave the branch out)
+          if (!kPar && p.out_u8) {
+            uint8_t* op = reinterpret_cast<uint8_t*>(outf_g) + o_off;
+            op[0] = (uint8_t)quant_u8(o0);
+            op[p.of_sc] = (uint8_t)quant_u8(o1);
+            op[2 * p.of_sc] = (uint8_t)quant_u8(o2);
+          } else {
+            float* op = outf_g + o_off;
+            op[0] = o0;
+            op[p.of_sc] = o1;
+            op[2 * p.of_sc] = o2;
+          }
         }
         cur = nxt;
         continue;

@@ -5,7 +5,8 @@
 //   ssim/_ssim (metrics.py:262-355): float64, 11x11 Gaussian window (sigma 1.5), valid part, mean of the map
 // on the host, after a device->host copy of every frame.  Here the frames never leave HBM: one kernel
 // accumulates the EXACT integer sum of squared uint8 differences per frame, one the float64 sum of the SSIM map
-// per frame and channel (separable 11-tap passes in shared memory).  Both are HBM-bound reads of 2 x 12 B/px.
+// per frame and channel (separable 11-tap passes in shared memory).  Both are HBM-bound reads of 2 x 12 B/px (fp32
+// frames) or 2 x 3 B/px (uint8 frames); each operand may be either, the kernels see the same uint8 values.
 #include <cstdint>
 
 #include "pnp_ops.cuh"
@@ -14,11 +15,10 @@ namespace pnp {
 
 namespace {
 
-__device__ __forceinline__ float quant_u8(float v) {
-  // misc.py:55-56,69: clamp_(0,1); (v - 0) / (1 - 0); * 255.0; numpy round (half to even)
-  v = fminf(fmaxf(v, 0.0f), 1.0f);
-  return rintf(__fmul_rn(v, 255.0f));
-}
+// One sample of an operand as tensor2img's uint8 value: fp32 frames are quantised (quant_u8), uint8 frames already hold
+// that value.  Either way the kernels below see the same float, so the results do not depend on the operand types.
+__device__ __forceinline__ float sample_u8(const float* p) { return quant_u8(__ldg(p)); }
+__device__ __forceinline__ float sample_u8(const uint8_t* p) { return (float)__ldg(p); }
 
 struct Gauss11 {
   double g[11];
@@ -26,9 +26,10 @@ struct Gauss11 {
 
 constexpr int kTileX = 32, kTileY = 8, kWinX = kTileX + 10, kWinY = kTileY + 10;
 
+template <typename TA, typename TB>
 __global__ void __launch_bounds__(256)
-sse_u8_kernel(const float* __restrict__ a, long long a_sf, long long a_sc, long long a_sy,
-              const float* __restrict__ b, long long b_sf, long long b_sc, long long b_sy, int H, int W, int crop,
+sse_u8_kernel(const TA* __restrict__ a, long long a_sf, long long a_sc, long long a_sy,
+              const TB* __restrict__ b, long long b_sf, long long b_sc, long long b_sy, int H, int W, int crop,
               unsigned long long* __restrict__ sse) {
   const int f = blockIdx.y;
   const int hc = H - 2 * crop, wc = W - 2 * crop;
@@ -38,8 +39,8 @@ sse_u8_kernel(const float* __restrict__ a, long long a_sf, long long a_sc, long 
     const int x = (int)(i % wc);
     const long long r = i / wc;
     const int y = (int)(r % hc), c = (int)(r / hc);
-    const float va = quant_u8(__ldg(a + f * a_sf + c * a_sc + (long long)(y + crop) * a_sy + x + crop));
-    const float vb = quant_u8(__ldg(b + f * b_sf + c * b_sc + (long long)(y + crop) * b_sy + x + crop));
+    const float va = sample_u8(a + f * a_sf + c * a_sc + (long long)(y + crop) * a_sy + x + crop);
+    const float vb = sample_u8(b + f * b_sf + c * b_sc + (long long)(y + crop) * b_sy + x + crop);
     const int d = (int)va - (int)vb;
     acc += (unsigned long long)(d * d);
   }
@@ -56,9 +57,10 @@ sse_u8_kernel(const float* __restrict__ a, long long a_sf, long long a_sc, long 
 }
 
 // grid (tiles_x, tiles_y, F * n_ch); ssim_sum[f * 3 + k] accumulates channel ch_first + k
+template <typename TA, typename TB>
 __global__ void __launch_bounds__(256)
-ssim_sum_kernel(const float* __restrict__ a, long long a_sf, long long a_sc, long long a_sy,
-                const float* __restrict__ b, long long b_sf, long long b_sc, long long b_sy, int H, int W, int crop,
+ssim_sum_kernel(const TA* __restrict__ a, long long a_sf, long long a_sc, long long a_sy,
+                const TB* __restrict__ b, long long b_sf, long long b_sc, long long b_sy, int H, int W, int crop,
                 int ch_first, int n_ch, const Gauss11 gk, double* __restrict__ ssim_sum) {
   __shared__ float sa[kWinY][kWinX], sb[kWinY][kWinX];
   __shared__ double hs[5][kWinY][kTileX];
@@ -67,15 +69,15 @@ ssim_sum_kernel(const float* __restrict__ a, long long a_sf, long long a_sc, lon
   const int hc = H - 2 * crop, wc = W - 2 * crop;          // cropped image
   const int hv = hc - 10, wv = wc - 10;                    // valid window positions
   const int x0 = blockIdx.x * kTileX, y0 = blockIdx.y * kTileY;
-  const float* pa = a + f * a_sf + c * a_sc;
-  const float* pb = b + f * b_sf + c * b_sc;
+  const TA* pa = a + f * a_sf + c * a_sc;
+  const TB* pb = b + f * b_sf + c * b_sc;
   for (int i = threadIdx.x; i < kWinY * kWinX; i += 256) {
     const int wy = i / kWinX, wx = i % kWinX;
     const int y = y0 + wy, x = x0 + wx;
     float va = 0.f, vb = 0.f;
     if (y < hc && x < wc) {
-      va = quant_u8(__ldg(pa + (long long)(y + crop) * a_sy + x + crop));
-      vb = quant_u8(__ldg(pb + (long long)(y + crop) * b_sy + x + crop));
+      va = sample_u8(pa + (long long)(y + crop) * a_sy + x + crop);
+      vb = sample_u8(pb + (long long)(y + crop) * b_sy + x + crop);
     }
     sa[wy][wx] = va;
     sb[wy][wx] = vb;
@@ -127,28 +129,40 @@ ssim_sum_kernel(const float* __restrict__ a, long long a_sf, long long a_sc, lon
   }
 }
 
-}  // namespace
-
-cudaError_t launch_frame_quality(const float* a, long long a_sf, long long a_sc, long long a_sy, const float* b,
-                                 long long b_sf, long long b_sc, long long b_sy, int F, int H, int W, int crop,
-                                 int ch_first, int n_ch, const double* gauss11, unsigned long long* sse,
-                                 double* ssim_sum, int num_sms, cudaStream_t stream) {
-  cudaError_t e = cudaMemsetAsync(sse, 0, sizeof(unsigned long long) * F, stream);
-  if (e != cudaSuccess) return e;
-  e = cudaMemsetAsync(ssim_sum, 0, sizeof(double) * 3 * F, stream);
-  if (e != cudaSuccess) return e;
+template <typename TA, typename TB>
+void launch_quality_kernels(const void* a, long long a_sf, long long a_sc, long long a_sy, const void* b, long long b_sf,
+                            long long b_sc, long long b_sy, int F, int H, int W, int crop, int ch_first, int n_ch,
+                            const Gauss11& gk, unsigned long long* sse, double* ssim_sum, int num_sms,
+                            cudaStream_t stream) {
+  const TA* pa = static_cast<const TA*>(a);
+  const TB* pb = static_cast<const TB*>(b);
   const int hc = H - 2 * crop, wc = W - 2 * crop;
   const long long total = 3LL * hc * wc;
   int blocks = (int)((total + 256 * 8 - 1) / (256 * 8));
   if (blocks > 4 * num_sms) blocks = 4 * num_sms;
   if (blocks < 1) blocks = 1;
-  sse_u8_kernel<<<dim3(blocks, F), 256, 0, stream>>>(a, a_sf, a_sc, a_sy, b, b_sf, b_sc, b_sy, H, W, crop, sse);
-  Gauss11 gk;
-  for (int i = 0; i < 11; ++i) gk.g[i] = gauss11[i];
+  sse_u8_kernel<TA, TB><<<dim3(blocks, F), 256, 0, stream>>>(pa, a_sf, a_sc, a_sy, pb, b_sf, b_sc, b_sy, H, W, crop, sse);
   const int hv = hc - 10, wv = wc - 10;
   dim3 grid((wv + kTileX - 1) / kTileX, (hv + kTileY - 1) / kTileY, F * n_ch);
-  ssim_sum_kernel<<<grid, 256, 0, stream>>>(a, a_sf, a_sc, a_sy, b, b_sf, b_sc, b_sy, H, W, crop, ch_first, n_ch, gk,
-                                            ssim_sum);
+  ssim_sum_kernel<TA, TB><<<grid, 256, 0, stream>>>(pa, a_sf, a_sc, a_sy, pb, b_sf, b_sc, b_sy, H, W, crop, ch_first,
+                                                    n_ch, gk, ssim_sum);
+}
+
+}  // namespace
+
+cudaError_t launch_frame_quality(const void* a, bool a_u8, long long a_sf, long long a_sc, long long a_sy,
+                                 const void* b, bool b_u8, long long b_sf, long long b_sc, long long b_sy, int F, int H,
+                                 int W, int crop, int ch_first, int n_ch, const double* gauss11,
+                                 unsigned long long* sse, double* ssim_sum, int num_sms, cudaStream_t stream) {
+  cudaError_t e = cudaMemsetAsync(sse, 0, sizeof(unsigned long long) * F, stream);
+  if (e != cudaSuccess) return e;
+  e = cudaMemsetAsync(ssim_sum, 0, sizeof(double) * 3 * F, stream);
+  if (e != cudaSuccess) return e;
+  Gauss11 gk;
+  for (int i = 0; i < 11; ++i) gk.g[i] = gauss11[i];
+  auto run = a_u8 ? (b_u8 ? launch_quality_kernels<uint8_t, uint8_t> : launch_quality_kernels<uint8_t, float>)
+                  : (b_u8 ? launch_quality_kernels<float, uint8_t> : launch_quality_kernels<float, float>);
+  run(a, a_sf, a_sc, a_sy, b, b_sf, b_sc, b_sy, F, H, W, crop, ch_first, n_ch, gk, sse, ssim_sum, num_sms, stream);
   return cudaGetLastError();
 }
 

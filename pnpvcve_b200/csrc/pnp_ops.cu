@@ -339,6 +339,40 @@ cudaError_t launch_lr_im2col(const float* lr, long long sn, long long sc, long l
 }
 
 // =====================================================================================
+// 8-bit frames -> the reference's fp32 lq: RescaleToZeroOne computes img.astype(np.float32) / 255. (normalization.py:
+// 93-99), a correctly rounded fp32 division.  Multiplying by fl(1/255) instead differs for 126 of the 256 values, so
+// the value table is built with __fdiv_rn.  HBM-bound (3 B in, 12 B out per pixel); kept out of lr_im2col and the
+// conv_last epilogue, which read the fp32 frame: what fusing would save is ~14 MB per 720p frame against ~10 GB of
+// feature traffic.
+// =====================================================================================
+constexpr int kU8PerThread = 4;
+__global__ void __launch_bounds__(256)
+unit_from_u8_kernel(const uint8_t* __restrict__ src, long long s_sf, long long s_sc, long long s_sy,
+                    float* __restrict__ dst, long long d_sf, long long d_sc, long long d_sy, int H, int W) {
+  __shared__ float lut[256];
+  lut[threadIdx.x] = __fdiv_rn((float)threadIdx.x, 255.0f);
+  __syncthreads();
+  const int f = blockIdx.z, c = blockIdx.y / H, y = blockIdx.y % H;
+  const uint8_t* s = src + f * s_sf + c * s_sc + y * s_sy;
+  float* d = dst + f * d_sf + c * d_sc + y * d_sy;
+  const int x0 = blockIdx.x * (256 * kU8PerThread) + threadIdx.x;
+#pragma unroll
+  for (int k = 0; k < kU8PerThread; ++k) {
+    const int x = x0 + k * 256;
+    if (x < W) d[x] = lut[__ldg(s + x)];
+  }
+}
+
+cudaError_t launch_unit_from_u8(const uint8_t* src, long long s_sf, long long s_sc, long long s_sy, float* dst,
+                               long long d_sf, long long d_sc, long long d_sy, int F, int H, int W,
+                               cudaStream_t stream) {
+  if (3LL * H > 65535 || F > 65535) return cudaErrorInvalidValue;
+  dim3 grid((W + 256 * kU8PerThread - 1) / (256 * kU8PerThread), 3 * H, F);
+  unit_from_u8_kernel<<<grid, 256, 0, stream>>>(src, s_sf, s_sc, s_sy, dst, d_sf, d_sc, d_sy, H, W);
+  return cudaGetLastError();
+}
+
+// =====================================================================================
 // Launch-table upload without the copy engine: the kernel reads PINNED host memory over the bus itself.  A
 // cudaMemcpyAsync of the (small) table queues behind whatever the H2D copy engine is already moving -- with clips
 // streaming in (driver.ClipStreamer) that is up to a whole clip, 67 ms at 720p x 100 frames, during which the first

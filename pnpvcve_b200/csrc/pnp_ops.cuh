@@ -10,6 +10,14 @@ struct DynRef;
 
 constexpr int kPackBlockBytes = 8192;
 
+// tensor2img's quantisation of one sample (mmedit/core/misc.py:55-56,69): clamp_(0,1); (v - 0) / (1 - 0); * 255.0;
+// numpy round (half to even).  Returns the uint8 value as a float.  Shared by the metrics and the uint8 store of
+// conv_last, so that a uint8 frame is exactly what quantising the fp32 frame gives.
+__device__ __forceinline__ float quant_u8(float v) {
+  v = fminf(fmaxf(v, 0.0f), 1.0f);
+  return rintf(__fmul_rn(v, 255.0f));
+}
+
 // tm_src / tm_dst: (64, W, H, images) bf16 maps of the source / destination buffer, boxes (64, 10, 10, 1) / (64, 8, 8, 1),
 // 128B swizzle, zero fill; table mode: both span the pool that starts at pool_base and the entry's pointers select the
 // images
@@ -38,10 +46,15 @@ cudaError_t launch_mix_bias(const float* conv2_bias, long long block_stride, int
                             const float* experts, const float* gamma, int frames, float* out,
                             cudaStream_t stream);
 
-cudaError_t launch_frame_quality(const float* a, long long a_sf, long long a_sc, long long a_sy, const float* b,
-                                 long long b_sf, long long b_sc, long long b_sy, int F, int H, int W, int crop,
-                                 int ch_first, int n_ch, const double* gauss11, unsigned long long* sse,
-                                 double* ssim_sum, int num_sms, cudaStream_t stream);
+cudaError_t launch_unit_from_u8(const uint8_t* src, long long s_sf, long long s_sc, long long s_sy, float* dst,
+                               long long d_sf, long long d_sc, long long d_sy, int F, int H, int W,
+                               cudaStream_t stream);
+
+// a_u8 / b_u8: the operand is a uint8 frame (read as is) instead of an fp32 one (quantised with quant_u8)
+cudaError_t launch_frame_quality(const void* a, bool a_u8, long long a_sf, long long a_sc, long long a_sy,
+                                 const void* b, bool b_u8, long long b_sf, long long b_sc, long long b_sy, int F, int H,
+                                 int W, int crop, int ch_first, int n_ch, const double* gauss11,
+                                 unsigned long long* sse, double* ssim_sum, int num_sms, cudaStream_t stream);
 
 cudaError_t launch_mv_rasterize(const float* rec, const int* frame_off, const int* is_b, const int* p_target,
                                 int T, int R, int H, int W, unsigned* own_f, unsigned* own_b, unsigned* pmask,

@@ -24,9 +24,16 @@ def clips_per_rank(num_clips, world):
     return (num_clips + world - 1) // world
 
 
+def _unit(x):
+    """Frames in [0,1] units: 8-bit frames as float32(v) / 255 (the loader's RescaleToZeroOne), others as they are."""
+    return x.float() / 255.0 if x.dtype == torch.uint8 else x
+
+
 def frame_metrics(out, ref=None):
-    """out (n,T,3,H,W) -> (n,T,N_METRICS) fp32 on the same device (no host sync)."""
-    d = out.float() if ref is None else (out - ref).float()
+    """out (n,T,3,H,W) -> (n,T,N_METRICS) fp32 on the same device (no host sync).  uint8 frames (out or ref) are
+    compared in [0,1] units, so max-abs and mse mean the same for fp32 and 8-bit frames."""
+    out = _unit(out)
+    d = out.float() if ref is None else (out - _unit(ref)).float()
     return torch.stack([d.abs().amax(dim=(2, 3, 4)), (d * d).mean(dim=(2, 3, 4))], dim=-1)
 
 
@@ -55,7 +62,7 @@ def gather_metrics(local, num_clips, rank, world, group=None):
 
 @torch.no_grad()
 def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=0, device=None, out_hosts=None,
-                  chunk=10):
+                  chunk=10, out_dtype=torch.float32):
     """Run this rank's share of ``clips``: a list of clip dicts as produced by pnpvcve_b200.synthetic, each holding
     n >= 1 equally shaped clips (n, T, ...); entries of other ranks may be None.
 
@@ -68,9 +75,20 @@ def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=
     (mmedit/models/restorers/basicvsr.py:119-153), but on the device (pnpvcve_b200.metrics) -- the reference's test loop
     copies every frame to the host and pickles per-clip results through two all_gathers (mmedit/apis/test.py:190-234);
     here nothing but the frames themselves leaves the GPU before the single fixed-shape gather.
+
+    8-bit frames: ``lq`` may be uint8 (value v stands for float32(v) / 255, what the reference's loader makes of a PNG),
+    and ``out_dtype=torch.uint8`` returns tensor2img's uint8 frames (mmedit/core/misc.py:9-74) of the fp32 result,
+    stored by the last conv itself -- same (n,T,3,H,W) layout, a quarter of the bytes over the bus and in pinned
+    memory.  ``out_hosts`` must then be uint8; ``gts`` / ``refs`` may be uint8 too.
     """
     from .synthetic import generator_args
     from . import metrics as _metrics
+    if out_dtype not in (torch.float32, torch.uint8):
+        raise ValueError(f"out_dtype must be torch.float32 or torch.uint8, got {out_dtype}")
+    if out_hosts is not None:
+        bad = [c for c, o in enumerate(out_hosts) if o is not None and o.dtype != out_dtype]
+        if bad:
+            raise ValueError(f"out_hosts[{bad[0]}] is {out_hosts[bad[0]].dtype}, out_dtype is {out_dtype}")
     mine = shard_clips(len(clips), rank, world)
     first = next(c for c in clips if c is not None)["lq"]
     shape_of = first.shape
@@ -96,7 +114,7 @@ def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=
         ticket = streamer.upload(pinned[mine[0]])
         for i, c in enumerate(mine):
             dst = out_hosts[c] if out_hosts is not None else \
-                torch.empty((n, t, 3, shape_of[-2] * up, shape_of[-1] * up), dtype=torch.float32).pin_memory()
+                torch.empty((n, t, 3, shape_of[-2] * up, shape_of[-1] * up), dtype=out_dtype).pin_memory()
             out = streamer.run(ticket, dst)
             ticket = streamer.upload(pinned[mine[i + 1]]) if i + 1 < len(mine) else None   # overlaps clip c's kernels
             measure(c, out)                 # on the device copy, before its buffer is recycled two entries later
@@ -104,7 +122,14 @@ def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=
         streamer.finish(check=True)
     else:
         for c in mine:
-            out = net(*generator_args(clips[c]))
+            if out_dtype == torch.uint8:
+                lq = clips[c]["lq"]
+                up = 4 if getattr(net, "vsr", False) else 1
+                buf = torch.empty(tuple(lq.shape[:3]) + ((lq.shape[3] + 3) // 4 * 4 * up, (lq.shape[4] + 3) // 4 * 4 * up),
+                                  dtype=torch.uint8, device=lq.device)
+                out = net.forward_streamed(*generator_args(clips[c]), out=buf)
+            else:
+                out = net(*generator_args(clips[c]))
             outs.append(out)
             measure(c, out)
     nm = N_METRICS + (2 if gts is not None else 0)
@@ -332,6 +357,9 @@ class ClipStreamer:
     def upload(self, host_clip):
         """Enqueue the upload of one clip; returns a ticket for ``run``.
 
+        8-bit frames: a uint8 ``lq`` is streamed as uint8 into a uint8 device copy; ``run`` dequantises each chunk into the
+        fp32 ``lq`` the kernels read as soon as it has arrived, on the kernels' stream.
+
         COMPACT side information: a host clip that carries ``side`` (a list of n ``sideinfo.pack_side`` dicts: the
         codec's per-block motion-vector records, 40 bytes per block) instead of the dense ``mvs`` / ``partitions``
         planes uploads those records and rasterises them on the device (``pnp_mv_rasterize``, the bit-exact
@@ -343,6 +371,7 @@ class ClipStreamer:
         side = host_clip.get("side")
         tensors = {k: v for k, v in host_clip.items() if k != "side"}
         n, _, _, h, w = host_clip["lq"].shape
+        lq_u8 = host_clip["lq"].dtype == torch.uint8
         if side is not None:
             if len(side) != n or any(sd["t"] != t for sd in side):
                 raise ValueError(f"side information must hold one packed entry of {t} frames per clip ({n})")
@@ -350,7 +379,10 @@ class ClipStreamer:
                           mvs=((n, t, 4, h, w), torch.float32), partitions=((n, t, 3, h, w), torch.float32))
         else:
             shapes = {k: (tuple(v.shape), v.dtype) for k, v in tensors.items()}
-        key = tuple((k, sh) for k, (sh, _) in sorted(shapes.items()))
+        if lq_u8:                          # the uint8 chunks land in lq_u8, the kernels read the fp32 lq
+            shapes["lq_u8"] = shapes["lq"]
+            shapes["lq"] = (shapes["lq"][0], torch.float32)
+        key = tuple((k, sh, dt) for k, (sh, dt) in sorted(shapes.items()))
         if self.slots[slot] is None or self.slots[slot][0] != key:
             self.slots[slot] = (key, {k: torch.empty(sh, dtype=dt, device=self.dev) for k, (sh, dt) in shapes.items()},
                                 None)
@@ -377,29 +409,42 @@ class ClipStreamer:
             big = [k for k in self.BIG if k in tensors]
             for a, b in reversed(self._chunks(t)):
                 for k in big if self.copy_in else ():
+                    dk = "lq_u8" if (k == "lq" and lq_u8) else k
                     for c in range(n):
-                        dclip[k][c, a:b].copy_(host_clip[k][c, a:b], non_blocking=True)
+                        dclip[dk][c, a:b].copy_(host_clip[k][c, a:b], non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record(self.up)
                 events[(a, b)] = ev
         self.h2d_bytes = sum(v.numel() * v.element_size() for v in tensors.values()) + side_bytes
-        return dict(slot=slot, dclip=dclip, events=events, t=t, side_dev=side_dev, side_ev=side_ev,
+        return dict(slot=slot, dclip=dclip, events=events, t=t, side_dev=side_dev, side_ev=side_ev, lq_u8=lq_u8,
                     cond=(host_clip["slices"], host_clip["base_QPs"], host_clip["QPs"]))
 
     @torch.no_grad()
     def run(self, ticket, out_host):
-        """Enqueue the kernels of an uploaded clip and the chunked download of its frames into ``out_host``."""
+        """Enqueue the kernels of an uploaded clip and the chunked download of its frames into ``out_host`` (fp32, or
+        uint8: the last conv then stores tensor2img's uint8 frames)."""
         main = torch.cuda.current_stream(self.dev)
         t, dclip, events = ticket["t"], ticket["dclip"], ticket["events"]
         chunks = self._chunks(t)
         owner = self._chunk_of(chunks, t)
         waited = set()
 
+        def arrive(ch):
+            """the kernels' stream waits for chunk ``ch``; 8-bit frames are then dequantised there (on the copy stream
+            the kernel would share the SMs with the previous clip's persistent conv kernels)"""
+            waited.add(ch)
+            main.wait_event(events[ch])
+            if ticket["lq_u8"]:
+                from . import ops
+                a, b = ch
+                with torch.cuda.device(self.dev):
+                    for c in range(dclip["lq"].shape[0]):
+                        ops.unit_from_u8(dclip["lq_u8"][c, a:b], dclip["lq"][c, a:b])
+
         def frame_ready(i):
             c = owner[i]
             if c not in waited:
-                waited.add(c)
-                main.wait_event(events[c])
+                arrive(c)
 
         def frame_done(i, out):
             a, b = owner[i]
@@ -411,8 +456,7 @@ class ClipStreamer:
                     for c in range(out.shape[0]) if self.copy_out else ():
                         out_host[c, a:b].copy_(out[c, a:b], non_blocking=True)
 
-        main.wait_event(events[chunks[-1]])          # small tensors + the first chunk the kernels need
-        waited.add(chunks[-1])
+        arrive(chunks[-1])                           # small tensors + the first chunk the kernels need
         if ticket["side_dev"]:
             # compact side information: records -> dense mvs / partitions of the whole clip, ahead of its first kernel
             # (~47 us per 720p frame).  The planes' previous readers ran on this stream, so plain stream order suffices.
@@ -434,12 +478,12 @@ class ClipStreamer:
         # result buffers are owned here and recycled under events: a fresh torch.empty per clip that another stream
         # still reads (record_stream) keeps the caching allocator from reusing the block and ends in cudaMalloc stalls
         slot = ticket["slot"]
-        if self.outs[slot] is not None and tuple(self.outs[slot][0].shape[:2]) == tuple(out_host.shape[:2]) and \
-                tuple(self.outs[slot][0].shape[2:]) == tuple(out_host.shape[2:]):
+        if self.outs[slot] is not None and tuple(self.outs[slot][0].shape) == tuple(out_host.shape) and \
+                self.outs[slot][0].dtype == out_host.dtype:
             obuf, free_ev = self.outs[slot]
             main.wait_event(free_ev)
         else:
-            obuf = torch.empty(out_host.shape, dtype=torch.float32, device=self.dev)
+            obuf = torch.empty(out_host.shape, dtype=out_host.dtype, device=self.dev)
         out = self.net.forward_streamed(*generator_args(dclip), cond_host=ticket["cond"], frame_ready=frame_ready,
                                         frame_done=frame_done, out=obuf)
         free_ev = torch.cuda.Event()

@@ -119,7 +119,7 @@ class _Program:
         self.stride = 8 + 2 * nb + (8 if vsr else 0)              # launch-table entries per step
         self.table_steps = 0
         self.table = self.img_off = self.host_table = self.host_off = None
-        self.nodes = {}          # (variant, nn, per_image, sparse) -> [(kind, label, args)]
+        self.nodes = {}          # (variant, nn, per_image, sparse, out_u8) -> [(kind, label, args)]
         self.graphs = {}         # same key -> graph handle
         self.ensure_table(table_steps)
         self.step_word = torch.zeros(1, dtype=torch.int32, device=dev)
@@ -319,9 +319,10 @@ class BaeEngine:
         self.prog.ensure_table(steps)
         return self.prog
 
-    def _build_nodes(self, pg, variant, nn, per_image, sparse, shapes):
+    def _build_nodes(self, pg, variant, nn, per_image, sparse, shapes, out_u8=False):
         """Launch sequence of one step variant for a run of ``nn`` clips: [(kind, label, ctypes args)], every operand
-        that changes per step left to the launch table (node index = position in the list)."""
+        that changes per step left to the launch table (node index = position in the list).  out_u8: conv_last stores
+        uint8 frames (the descriptor, and with it a captured graph, differs)."""
         lib = _lib.load()
         nodes = []
         h, w, nb = pg.h, pg.w, pg.nb
@@ -358,6 +359,7 @@ class BaeEngine:
                 d.lq, d.outf = 1, 1
                 d.lq_sn, d.lq_sc, d.lq_sy = shapes["lq"]       # with lq_up4: strides of the LR frame itself
                 d.of_sn, d.of_sc, d.of_sy = shapes["outf"]
+                d.out_u8 = 1 if out_u8 else 0
             d.N, d.H, d.W = nn, hh, ww
             d.tap_n = 16 if last else 64
             d.aux_k16 = 2 if aux else 0
@@ -437,7 +439,7 @@ class BaeEngine:
         plane = h * w * 4
         lr_ptr = ptrs["lrs"] + (b0 * t + frame) * 3 * plane
         par_ptr = ptrs["par"] + (b0 * t + frame) * 3 * plane
-        outf_ptr = ptrs["out"] + (b0 * t + frame) * 3 * plane * up * up
+        outf_ptr = ptrs["out"] + (b0 * t + frame) * 3 * h * w * up * up * ptrs["out_elem"]    # fp32 or uint8 frames
         mv_base = ptrs["mvs"] + (b0 * t + frame) * 4 * plane
         flow_x = np.where(steps < t, mv_base + 2 * plane, mv_base)               # bwd pass: channels 2,3; fwd: 0,1
         bias_row = 2 * nb * 64
@@ -550,7 +552,10 @@ class BaeEngine:
         frame_ready(i): called (host side) before frame i's lq / mvs / par_map are first read, in the backward-time
         pass (i = T-1 .. 0); frame_done(i, out): called after frame i's output has been enqueued.  Both let a caller
         stream a clip in and out in chunks (driver.ClipStreamer): they typically enqueue an event wait / record.
-        out: optional preallocated fp32 (n,T,3,Hout,Wout) result buffer (the caller guarantees nobody still reads it)."""
+        out: optional preallocated fp32 (n,T,3,Hout,Wout) result buffer (the caller guarantees nobody still reads it),
+        or a uint8 one: conv_last then stores tensor2img's uint8 value of every output sample.
+        lrs may be uint8 8-bit frames: value v stands for float32(v) / 255 (the reference loader's RescaleToZeroOne);
+        the clip is dequantised into an fp32 device tensor first."""
         m = self.m
         dev = lrs.device
         lib = _lib.load()
@@ -559,11 +564,19 @@ class BaeEngine:
         assert h_in >= 64 and w_in >= 64, (
             f"The height and width of inputs should be at least 64, but got {h_in} and {w_in}.")
         pad_h, pad_w = (4 - h_in % 4) % 4, (4 - w_in % 4) % 4
-        if frame_ready is not None and (pad_h or pad_w or not (lrs.is_contiguous() and mvs.is_contiguous()
-                                                              and par_map.is_contiguous())):
+        lq_u8 = lrs.dtype == torch.uint8
+        if frame_ready is not None and (pad_h or pad_w or lq_u8 or not (lrs.is_contiguous() and mvs.is_contiguous()
+                                                                       and par_map.is_contiguous())):
             for i in range(t):                            # whole-tensor copies below: everything must have arrived
                 frame_ready(i)
             frame_ready = None
+        if lq_u8:                                         # 8-bit frames: v / 255 in fp32, before the reflect padding
+            src = lrs if lrs.stride(-1) == 1 else lrs.contiguous()
+            try:
+                src.view(n * t, c, h_in, w_in)
+            except RuntimeError:
+                src = src.contiguous()
+            lrs = ops.unit_from_u8(src, torch.empty(lrs.shape, dtype=torch.float32, device=dev))
         if pad_h or pad_w:                                # spatial_padding, iconvsr.py:371-394
             lrs = F.pad(lrs.reshape(-1, c, h_in, w_in), [0, pad_w, 0, pad_h], mode="reflect")
             lrs = lrs.view(n, t, c, h_in + pad_h, w_in + pad_w)
@@ -608,9 +621,10 @@ class BaeEngine:
         up = 4 if m.vsr else 1
         if out is None:
             out = torch.empty((n, t, 3, up * h, up * w), dtype=torch.float32, device=dev)
-        elif tuple(out.shape) != (n, t, 3, up * h, up * w) or out.dtype != torch.float32 or out.device != dev or \
-                not out.is_contiguous():
-            raise ValueError(f"out must be a contiguous fp32 {(n, t, 3, up * h, up * w)} tensor on {dev}")
+        elif tuple(out.shape) != (n, t, 3, up * h, up * w) or out.dtype not in (torch.float32, torch.uint8) or \
+                out.device != dev or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous fp32 or uint8 {(n, t, 3, up * h, up * w)} tensor on {dev}")
+        out_u8 = out.dtype == torch.uint8
         feats = pg.feats
         bwd_feats = torch.empty_like(feats) if return_features else None
         # the reference takes the sparse path only in eval mode (sr_backbone_utils.py:307: `self.sparse_val and
@@ -621,7 +635,7 @@ class BaeEngine:
         if pg.uploaded is not None:
             pg.uploaded.synchronize()                     # the pinned staging buffers are reused between calls
         ptrs = dict(lrs=lrs.data_ptr(), par=par_map.data_ptr(), mvs=mvs.data_ptr(), out=out.data_ptr(),
-                    bias_tab=bias_tab.data_ptr())
+                    out_elem=out.element_size(), bias_tab=bias_tab.data_ptr())
         plans = []
         for g_idx, (b0, b1) in enumerate(groups):
             bwd_key, fwd_key = key_schedule(key_rows[b0])
@@ -678,10 +692,10 @@ class BaeEngine:
 
         def run_step(step, variant, nn, per_image):
             nonlocal launches
-            key = (variant, nn, per_image, sparse)
+            key = (variant, nn, per_image, sparse, out_u8)      # a captured graph bakes in the descriptors
             nodes = pg.nodes.get(key)
             if nodes is None:
-                nodes = pg.nodes[key] = self._build_nodes(pg, variant, nn, per_image, sparse, shapes)
+                nodes = pg.nodes[key] = self._build_nodes(pg, variant, nn, per_image, sparse, shapes, out_u8)
             launches += len(nodes)
             if not graphs:
                 _lib.check(lib.pnp_set_step(step_ptr, step, stream), "pnp_set_step")

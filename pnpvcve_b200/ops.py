@@ -56,6 +56,37 @@ def _plane_view_check(t, name):
         raise ValueError(f"{name} must be an fp32 CUDA view with unit innermost stride")
 
 
+def _frames_view(t, name, dtype):
+    """(F,3,H,W) view of a (F,3,H,W) or (n,T,3,H,W) frame tensor of ``dtype`` with unit innermost stride."""
+    if t.dtype != dtype or not t.is_cuda or t.dim() not in (4, 5) or t.shape[-3] != 3 or t.stride(-1) != 1:
+        raise ValueError(f"{name} must be a {dtype} CUDA (F,3,H,W) or (n,T,3,H,W) view with unit innermost stride, got "
+                         f"{tuple(t.shape)} {t.dtype}")
+    if t.dim() == 5:
+        try:
+            t = t.view(-1, *t.shape[2:])
+        except RuntimeError:
+            raise ValueError(f"{name}: the (n,T) dimensions of a 5-D view must merge into one frame stride") from None
+    return t
+
+
+@_on_device_of
+def unit_from_u8(src_u8, dst_f32):
+    """8-bit frames -> fp32 frames in [0,1]: dst = float32(v) / 255, correctly rounded (the reference loader's
+    ``img.astype(np.float32) / 255.``).  src_u8 uint8 and dst_f32 fp32 views of the same (F,3,H,W) or (n,T,3,H,W) shape,
+    unit innermost stride."""
+    if src_u8.shape != dst_f32.shape:
+        raise ValueError(f"unit_from_u8: shapes {tuple(src_u8.shape)} / {tuple(dst_f32.shape)} differ")
+    s = _frames_view(src_u8, "src_u8", torch.uint8)
+    d = _frames_view(dst_f32, "dst_f32", torch.float32)
+    if s.numel() == 0:
+        return dst_f32
+    f, _, h, w = s.shape
+    lib = _lib.load()
+    _lib.check(lib.pnp_unit_from_u8(_ptr(s), s.stride(0), s.stride(1), s.stride(2), _ptr(d), d.stride(0), d.stride(1),
+                                    d.stride(2), f, h, w, _stream()), "pnp_unit_from_u8")
+    return dst_f32
+
+
 def fetch_pinned(dst, src):
     """dst (device) <- src (pinned host tensor of the same byte size), stream ordered, WITHOUT the copy engine (the
     launch table must not queue behind a clip that is being uploaded)."""
@@ -230,9 +261,11 @@ def fill_conv_desc(d, src, wpack, out=None, aux=None, idt=None, scale=None, bias
         d.par, d.par_sn, d.par_sc, d.par_sy = par.data_ptr(), par.stride(0), par.stride(1), par.stride(2)
     else:
         d.par, d.par_sn, d.par_sc, d.par_sy = None, 0, 0, 0
+    d.out_u8 = 0
     if last:
         d.lq, d.lq_sn, d.lq_sc, d.lq_sy = lq.data_ptr(), lq.stride(0), lq.stride(1), lq.stride(2)
         d.outf, d.of_sn, d.of_sc, d.of_sy = outf.data_ptr(), outf.stride(0), outf.stride(1), outf.stride(2)
+        d.out_u8 = 1 if outf.dtype == torch.uint8 else 0
     else:
         d.lq, d.lq_sn, d.lq_sc, d.lq_sy = None, 0, 0, 0
         d.outf, d.of_sn, d.of_sc, d.of_sy = None, 0, 0, 0
@@ -258,7 +291,7 @@ def conv3x3(src, wpack, out=None, aux=None, idt=None, scale=None, bias=None, par
     """Fused tcgen05 3x3 conv (see include/pnp_vcve.h: pnp_conv3x3).  `out` may be a strided view with unit
     channel stride (pixel shuffle as the store epilogue); lq_up4: lq is the (N,3,H/4,W/4) frame whose x4
     bilinear upsampling is added; img_off: per-image weight / bias offsets (one launch, N differently
-    conditioned images)."""
+    conditioned images).  A uint8 `outf` receives tensor2img's uint8 values of the fp32 result (out_u8)."""
     _feat_check(src, "src")
     for t, nm in ((out, "out"), (idt, "idt")):
         if t is not None:
@@ -271,7 +304,11 @@ def conv3x3(src, wpack, out=None, aux=None, idt=None, scale=None, bias=None, par
             raise ValueError(f"conv3x3: aux shape {tuple(aux.shape)} does not match src {tuple(src.shape)}")
     for t, nm in ((par, "par"), (lq, "lq"), (outf, "outf")):
         if t is not None:
-            _plane_view_check(t, nm)
+            if nm == "outf" and t.dtype == torch.uint8:
+                if t.stride(-1) != 1 or not t.is_cuda:
+                    raise ValueError("outf must be a CUDA view with unit innermost stride")
+            else:
+                _plane_view_check(t, nm)
             hw = tuple(src.shape[1:3])
             if nm == "lq" and lq_up4:
                 hw = (src.shape[1] // 4, src.shape[2] // 4)
