@@ -179,6 +179,21 @@ int pnp_mv_rasterize(const float* records, const int32_t* frame_offsets, const i
                      const int32_t* p_target, int T, int R, int H, int W, uint32_t* owner_fwd,
                      uint32_t* owner_bwd, uint32_t* part_mask, float* mvs, float* partitions,
                      int32_t* status, void* stream);
+/* The planes of a frame window [a, b) of a clip, bit-identical to frames [a, b) of pnp_mv_rasterize on the whole clip
+ * (what the reference computes when it slices the dense tensors of a whole clip, restoration_video_inference.py:121-128).
+ * Only one later frame writes into the window: the TAIL frame e, the first non-B frame >= b, whose reversed records land
+ * in the previous non-B frame.  The table holds the window's frames, then at most one tail frame, in clip order:
+ *   records       : the records of frames [a, b), then (tail = 1) the direction>0 records of frame e
+ *   frame_offsets : int32 (T+tail+1), window-relative; is_b, p_target : int32 (T+tail), window-relative frame indices
+ *   p_target      : as above, plus -2 for a target before the window (the write is skipped, no status bit)
+ *   tail          : 0 or 1; a tail record makes only its reversed write (no forward write, no partition mark, no
+ *                   status bit 1: its frame lies outside the window, which owns none of its errors)
+ *   T, owner_fwd/owner_bwd/part_mask, mvs, partitions, status: as above, T = b - a window frames.
+ * An addition: the ABI version and every other entry point are unchanged. */
+int pnp_mv_rasterize_window(const float* records, const int32_t* frame_offsets, const int32_t* is_b,
+                            const int32_t* p_target, int T, int tail, int R, int H, int W, uint32_t* owner_fwd,
+                            uint32_t* owner_bwd, uint32_t* part_mask, float* mvs, float* partitions,
+                            int32_t* status, void* stream);
 
 /*
  * Per-frame quality metrics of the reference's test loop, computed where the frames are ("next" row of the scope

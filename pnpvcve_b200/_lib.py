@@ -21,7 +21,7 @@ EXPORTS = [
     "pnp_mv_warp", "pnp_mv_warp_dyn", "pnp_lr_im2col", "pnp_lr_im2col_dyn", "pnp_pack_conv3x3_rowstack",
     "pnp_pack_rows", "pnp_pack_aux", "pnp_pack_mix_blocks",
     "pnp_caa_heads", "pnp_mix_bias", "pnp_mv_rasterize", "pnp_conv3x3", "pnp_frame_quality", "pnp_frame_quality_u8",
-    "pnp_unit_from_u8",
+    "pnp_unit_from_u8", "pnp_mv_rasterize_window",
 ]
 
 _c = ctypes
@@ -80,6 +80,7 @@ _PROTOS = {
     "pnp_caa_heads": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "pnp_mix_bias": (_i, [_vp, _i, _i, _vp, _vp, _i, _vp, _vp]),
     "pnp_mv_rasterize": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pnp_mv_rasterize_window": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pnp_conv3x3": (_i, [_c.POINTER(ConvDesc), _vp]),
     "pnp_frame_quality": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pnp_frame_quality_u8": (_i, [_vp, _i, _i64, _i64, _i64, _vp, _i, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _vp, _vp]),

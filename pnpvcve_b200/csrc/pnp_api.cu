@@ -456,9 +456,29 @@ int pnp_mv_rasterize(const float* records, const int32_t* frame_offsets, const i
   DeviceInfo* d;
   int rc = device_info(&d);
   if (rc) return rc;
-  cudaError_t e = pnp::launch_mv_rasterize(records, frame_offsets, is_b, p_target, T, R, H, W, owner_fwd, owner_bwd,
-                                           part_mask, mvs, partitions, status, static_cast<cudaStream_t>(stream));
+  cudaError_t e = pnp::launch_mv_rasterize(records, frame_offsets, is_b, p_target, T, 0, false, R, H, W, owner_fwd,
+                                           owner_bwd, part_mask, mvs, partitions, status,
+                                           static_cast<cudaStream_t>(stream));
   return e == cudaSuccess ? PNP_OK : cuda_fail(e, "pnp_mv_rasterize");
+}
+
+int pnp_mv_rasterize_window(const float* records, const int32_t* frame_offsets, const int32_t* is_b,
+                            const int32_t* p_target, int T, int tail, int R, int H, int W, uint32_t* owner_fwd,
+                            uint32_t* owner_bwd, uint32_t* part_mask, float* mvs, float* partitions,
+                            int32_t* status, void* stream) {
+  if (!frame_offsets || !is_b || !p_target || !owner_fwd || !owner_bwd || !part_mask || !mvs || !partitions ||
+      !status || (R > 0 && !records))
+    return fail(PNP_ERR_ARG, "pnp_mv_rasterize_window: null pointer");
+  if (T < 1 || T > 65535 || (tail != 0 && tail != 1) || R < 0 || H < 1 || H > 65535 || W < 1 ||
+      (long long)T * H * W >= (1LL << 31))
+    return fail(PNP_ERR_ARG, "pnp_mv_rasterize_window: bad shape");
+  DeviceInfo* d;
+  int rc = device_info(&d);
+  if (rc) return rc;
+  cudaError_t e = pnp::launch_mv_rasterize(records, frame_offsets, is_b, p_target, T, tail, true, R, H, W, owner_fwd,
+                                           owner_bwd, part_mask, mvs, partitions, status,
+                                           static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? PNP_OK : cuda_fail(e, "pnp_mv_rasterize_window");
 }
 
 int pnp_frame_quality(const float* a, int64_t a_sf, int64_t a_sc, int64_t a_sy, const float* b, int64_t b_sf,

@@ -56,8 +56,10 @@ cudaError_t launch_frame_quality(const void* a, bool a_u8, long long a_sf, long 
                                  int W, int crop, int ch_first, int n_ch, const double* gauss11,
                                  unsigned long long* sse, double* ssim_sum, int num_sms, cudaStream_t stream);
 
+// window = false: a whole clip (tail must be 0, every negative p_target is an error); true: a frame window with `tail`
+// (0 / 1) tail frames after its T frames and p_target -2 for targets before the window
 cudaError_t launch_mv_rasterize(const float* rec, const int* frame_off, const int* is_b, const int* p_target,
-                                int T, int R, int H, int W, unsigned* own_f, unsigned* own_b, unsigned* pmask,
-                                float* mvs, float* partitions, int* status, cudaStream_t stream);
+                                int T, int tail, bool window, int R, int H, int W, unsigned* own_f, unsigned* own_b,
+                                unsigned* pmask, float* mvs, float* partitions, int* status, cudaStream_t stream);
 
 }  // namespace pnp

@@ -12,6 +12,11 @@
 //     direction>0 on a non-B frame -> NEGATED into channels 2,3 of the previous non-B frame at the
 //     SOURCE block position; direction==0 -> no motion write (the reference's assert is a no-op);
 //   * partition channel {256:0,128:1,64:2}[w*h] is set (never cleared) for every record.
+// A frame window [a, b) of a clip (pnp_mv_rasterize_window) gives the planes of frames [a, b) of the whole-clip result:
+// its table holds the window's records plus the reversed records of the tail frame e (the first non-B frame >= b, the
+// only later frame that writes into the window), in clip order, so record-order overwrite and the fill pass's negation
+// test hold unchanged.  A tail record makes only its reversed write; a target before the window (p_target -2) is
+// skipped.
 #include "pnp_ops.cuh"
 
 namespace pnp {
@@ -32,8 +37,9 @@ __device__ __forceinline__ void np_slice(int a, int b, int n, int& lo, int& hi) 
 
 __global__ void __launch_bounds__(256)
 raster_owner_kernel(const float* __restrict__ rec, const int* __restrict__ frame_off, const int* __restrict__ is_b,
-                    const int* __restrict__ p_target, int T, int R, int H, int W, unsigned* __restrict__ own_f,
-                    unsigned* __restrict__ own_b, unsigned* __restrict__ pmask, int* __restrict__ status) {
+                    const int* __restrict__ p_target, int T, int tail, int window, int R, int H, int W,
+                    unsigned* __restrict__ own_f, unsigned* __restrict__ own_b, unsigned* __restrict__ pmask,
+                    int* __restrict__ status) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= R) return;
@@ -43,13 +49,14 @@ raster_owner_kernel(const float* __restrict__ rec, const int* __restrict__ frame
   // frame of this record: last f with frame_off[f] <= warp
   int f = 0;
   {
-    int lo = 0, hi = T;                       // frame_off has T+1 entries
+    int lo = 0, hi = T + tail;                // frame_off has T+tail+1 entries
     while (hi - lo > 1) {
       const int mid = (lo + hi) >> 1;
       if (frame_off[mid] <= warp) lo = mid; else hi = mid;
     }
     f = lo;
   }
+  const bool in_tail = f == T;               // the tail frame's own planes lie outside the window
   const size_t plane = (size_t)H * W;
   const unsigned key = (unsigned)warp + 1u;   // global record index + 1: later records win
   // partition: every record, destination block
@@ -57,18 +64,20 @@ raster_owner_kernel(const float* __restrict__ rec, const int* __restrict__ frame
   np_slice(y - floordiv2(h), y + floordiv2(h), H, r0, r1);
   np_slice(x - floordiv2(w), x + floordiv2(w), W, c0, c1);
   const int area = w * h;
-  unsigned pbit = area == 256 ? 1u : area == 128 ? 2u : area == 64 ? 4u : 0u;
-  if (pbit == 0u && lane == 0) atomicOr(status, 1);          // KeyError in the reference
+  unsigned pbit = in_tail ? 0u : area == 256 ? 1u : area == 128 ? 2u : area == 64 ? 4u : 0u;
+  if (pbit == 0u && !in_tail && lane == 0) atomicOr(status, 1);   // KeyError in the reference
   unsigned* owner = nullptr;
   int tr0 = r0, tr1 = r1, tc0 = c0, tc1 = c1;
   if (direction < 0.f) {
-    owner = own_f + (size_t)f * plane;
+    if (!in_tail) owner = own_f + (size_t)f * plane;
   } else if (direction > 0.f) {
-    if (is_b[f]) {
+    if (!in_tail && is_b[f]) {                // (the tail frame is non-B)
       owner = own_b + (size_t)f * plane;
     } else {
       const int tgt = p_target[f];
-      if (tgt < 0) {
+      if (tgt == -2 && window) {
+        // target before the window: the write lands outside it
+      } else if (tgt < 0) {
         if (lane == 0) atomicOr(status, 2);                  // p_offset unbound / before the clip
       } else {
         owner = own_b + (size_t)tgt * plane;
@@ -140,12 +149,12 @@ raster_fill_kernel(const float* __restrict__ rec, const int* __restrict__ frame_
 }
 
 cudaError_t launch_mv_rasterize(const float* rec, const int* frame_off, const int* is_b, const int* p_target,
-                                int T, int R, int H, int W, unsigned* own_f, unsigned* own_b, unsigned* pmask,
-                                float* mvs, float* partitions, int* status, cudaStream_t stream) {
+                                int T, int tail, bool window, int R, int H, int W, unsigned* own_f, unsigned* own_b,
+                                unsigned* pmask, float* mvs, float* partitions, int* status, cudaStream_t stream) {
   if (R > 0) {
     const long long threads = (long long)R * 32;
-    raster_owner_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(rec, frame_off, is_b, p_target, T, R,
-                                                                             H, W, own_f, own_b, pmask, status);
+    raster_owner_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(
+        rec, frame_off, is_b, p_target, T, tail, window ? 1 : 0, R, H, W, own_f, own_b, pmask, status);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }

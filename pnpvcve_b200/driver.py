@@ -170,81 +170,116 @@ def clip_window(clip, a, b, overlap=0):
     [lo, hi) of the core frames [a, b) inside that window.  ``overlap`` > 0 runs extra context frames whose outputs are
     discarded: the forced key frames then sit ``overlap`` frames away from the frames that are kept, which bounds the
     seam error against the uncut clip at the price of (2 overlap / window) extra work.  overlap = 0 is the reference's
-    ``max_seq_len`` semantics exactly."""
+    ``max_seq_len`` semantics exactly.  Compact side information (``side``) is cut by ``sideinfo.window_side``: the
+    window's records plus the ones a later frame writes into it, new pinned host tensors."""
     t = clip["lq"].shape[1]
     a0, b0 = max(0, a - overlap), min(t, b + overlap)
-    return {k: v[:, a0:b0] for k, v in clip.items()}, a - a0, b - a0
+    win = {k: v[:, a0:b0] for k, v in clip.items() if k != "side"}
+    if "side" in clip:
+        from . import sideinfo
+        win["side"] = [sideinfo.window_side(sd, a0, b0) for sd in clip["side"]]
+    return win, a - a0, b - a0
+
+
+def _pinned(v):
+    """``v`` itself when it is already contiguous pinned memory (a window of a pinned clip is), else a pinned copy;
+    without a CUDA device (the CPU tests of the sharding logic) a contiguous one."""
+    if not torch.cuda.is_available():
+        return v.contiguous()
+    return v if v.is_contiguous() and v.is_pinned() else v.contiguous().pin_memory()
 
 
 @torch.no_grad()
 def enhance_windows(net, clips, window, rank=0, world=1, overlap=0, refs=None, gather_output=False, group=None,
-                    device=None, chunk=10):
+                    device=None, chunk=10, gts=None, crop_border=0, out_dtype=torch.float32):
     """Frame-window sharding (north_star: "sharding independent clips or frame windows per GPU"): the windows of
     ``clips`` (equally shaped (1,T,...) clip dicts) are dealt to the ranks round robin and enhanced independently.
-    HOST-resident clips stream their windows through ``ClipStreamer`` on ``device`` (only a rank's own windows ever
-    reach its GPU), device-resident clips are sliced in place.
+    HOST-resident clips stream their windows through the cached ``ClipStreamer`` of (net, device, chunk) on ``device``
+    (only a rank's own windows ever reach its GPU), device-resident clips are sliced in place.
+
+    A host clip may carry ``side`` (one ``sideinfo.pack_side`` entry of the whole clip) instead of the dense ``mvs`` /
+    ``partitions``: each rank uploads only the records of its own windows (``sideinfo.window_side``, overlap included)
+    and rasterises them on the device, bit-identical to the same frames of the whole clip's planes.  Device-resident
+    clips and stand-in callables take dense planes only.
+
+    8-bit frames: ``lq`` may be uint8, and ``out_dtype=torch.uint8`` returns tensor2img's uint8 frames, stored by the
+    last conv (as in ``enhance_clips``).  ``gts`` (per clip (1,T,3,H,W), fp32 or uint8) adds PSNR / SSIM
+    (``metrics.frame_quality`` with ``crop_border``) to every frame's metric vector: [max-abs, mse, PSNR, SSIM].
 
     Returns (outs, metrics): outs = {(clip, a, b): (1, b-a, 3, H, W) frames} of this rank's windows (device tensors)
     -- or, with ``gather_output``, the complete (num_clips, T, 3, H, W) result on every rank (one fixed-shape all_gather
-    of frames over NVLink) --, metrics = (num_clips, T, N_METRICS) of ALL frames on every rank (one fixed-shape
-    all_gather).  No collective touches the data path of a window."""
+    of frames over NVLink, in ``out_dtype``) --, metrics = (num_clips, T, M) of ALL frames on every rank (one
+    fixed-shape all_gather).  No collective touches the data path of a window."""
     from .synthetic import generator_args
+    from . import metrics as _metrics
+    if out_dtype not in (torch.float32, torch.uint8):
+        raise ValueError(f"out_dtype must be torch.float32 or torch.uint8, got {out_dtype}")
     num_clips = len(clips)
-    if any("side" in c for c in clips):
-        # a P frame's reversed records write into the previous non-B frame, which may lie in another window
-        raise ValueError("frame windows are cut from dense mvs / partitions planes; rasterise compact side information "
-                         "first (pnpvcve_b200.sideinfo.rasterize_clip)")
     t = clips[0]["lq"].shape[1]
     # host-resident clips are streamed when `net` is the generator (anything else -- a stand-in callable in the CPU tests
     # of the sharding logic -- is simply called on the tensors where they are)
     host = not clips[0]["lq"].is_cuda and hasattr(net, "forward_streamed")
+    if not host and any("side" in c for c in clips):
+        raise ValueError("frame windows of device-resident clips are cut from dense mvs / partitions planes; rasterise "
+                         "compact side information first (pnpvcve_b200.sideinfo.rasterize_clip) or pass host clips")
     dev = torch.device(device) if device is not None else \
         (torch.device("cuda", torch.cuda.current_device()) if host else clips[0]["lq"].device)
     mine = shard_windows(num_clips, t, window, rank, world)
+    up = 4 if getattr(net, "vsr", False) else 1
     outs = {}
-    local = torch.full((num_clips, t, N_METRICS), float("nan"), dtype=torch.float32, device=dev)
-    streamer, ticket, wins = None, None, []
+    nm = N_METRICS + (2 if gts is not None else 0)
+    local = torch.full((num_clips, t, nm), float("nan"), dtype=torch.float32, device=dev)
+    streamer, ticket, wins, dsts = None, None, [], {}
     if host and mine:
-        up = 4 if getattr(net, "vsr", False) else 1
-        streamer = ClipStreamer(net, dev, chunk=chunk)
-        for c, a, b in mine:          # contiguous pinned copies of this rank's windows (the clip itself may be pageable)
+        streamer = streamer_for(net, dev, chunk)
+        for c, a, b in mine:          # pinned windows of this rank (views when the clip itself is pinned)
             win, lo, hi = clip_window(clips[c], a, b, overlap)
-            wins.append(({k: v.contiguous().pin_memory() for k, v in win.items()}, lo, hi))
+            wins.append(({k: v if k == "side" else _pinned(v) for k, v in win.items()}, lo, hi))
         ticket = streamer.upload(wins[0][0])
     for i, (c, a, b) in enumerate(mine):
         if host:
             hwin, lo, hi = wins[i]
-            frames_w = hwin["lq"].shape[1]
-            dst = torch.empty((1, frames_w, 3, hwin["lq"].shape[-2] * up, hwin["lq"].shape[-1] * up),
-                              dtype=torch.float32).pin_memory()
-            full = streamer.run(ticket, dst)
+            shape = (1, hwin["lq"].shape[1], 3, hwin["lq"].shape[-2] * up, hwin["lq"].shape[-1] * up)
+            if shape not in dsts:     # one download target per window shape, written in stream order
+                dsts[shape] = _pinned(torch.empty(shape, dtype=out_dtype))
+            full = streamer.run(ticket, dsts[shape])
             ticket = streamer.upload(wins[i + 1][0]) if i + 1 < len(mine) else None
             out = full[:, lo:hi].clone()            # (the streamer recycles its device buffer two windows later)
         else:
             win, lo, hi = clip_window(clips[c], a, b, overlap)
-            out = net(*generator_args({k: v.contiguous() for k, v in win.items()}))[:, lo:hi]
+            args = generator_args({k: v.contiguous() for k, v in win.items()})
+            if out_dtype == torch.uint8:
+                lq = win["lq"]
+                buf = torch.empty(tuple(lq.shape[:3]) + ((lq.shape[3] + 3) // 4 * 4 * up, (lq.shape[4] + 3) // 4 * 4 * up),
+                                  dtype=torch.uint8, device=lq.device)
+                out = net.forward_streamed(*args, out=buf)[:, lo:hi]
+            else:
+                out = net(*args)[:, lo:hi]
         outs[(c, a, b)] = out
-        local[c, a:b] = frame_metrics(out, None if refs is None else refs[c][:, a:b].to(dev))[0]
+        m = frame_metrics(out, None if refs is None else refs[c][:, a:b].to(dev))[0]
+        if gts is not None:
+            q = _metrics.frame_quality(out, gts[c][:, a:b].to(dev), crop_border)
+            m = torch.cat([m, q["psnr"][0].float()[:, None], q["ssim"][0].float()[:, None]], dim=-1)
+        local[c, a:b] = m
     if streamer is not None:
-        streamer.finish()
+        streamer.finish(check=True)
     metrics = merge_sharded(local, world, group)
     if not gather_output:
         return outs, metrics
     # frames: every rank contributes ONLY its own windows, packed into a fixed (items, window, 3, H, W) block
-    up = 4 if getattr(net, "vsr", False) else 1
     h, w = clips[0]["lq"].shape[-2] * up, clips[0]["lq"].shape[-1] * up
     items_all = [shard_windows(num_clips, t, window, r, world) for r in range(world)]
     max_items = max(len(it) for it in items_all)
     wlen = min(window, t)
-    block = torch.zeros((max_items, wlen, 3, h, w), dtype=torch.float32, device=dev)
+    block = torch.zeros((max_items, wlen, 3, h, w), dtype=out_dtype, device=dev)
     for i, (c, a, b) in enumerate(mine):
         block[i, :b - a] = outs[(c, a, b)][0]
     if world == 1:
         parts = block[None]
     else:
-        parts = torch.empty((world,) + tuple(block.shape), dtype=torch.float32, device=dev)
+        parts = torch.empty((world,) + tuple(block.shape), dtype=out_dtype, device=dev)
         dist.all_gather(list(parts.unbind(0)), block, group=group)
-    frames = torch.empty((num_clips, t, 3, h, w), dtype=torch.float32, device=dev)
+    frames = torch.empty((num_clips, t, 3, h, w), dtype=out_dtype, device=dev)
     for r in range(world):
         for i, (c, a, b) in enumerate(items_all[r]):
             frames[c, a:b] = parts[r, i, :b - a]
@@ -364,7 +399,8 @@ class ClipStreamer:
         codec's per-block motion-vector records, 40 bytes per block) instead of the dense ``mvs`` / ``partitions``
         planes uploads those records and rasterises them on the device (``pnp_mv_rasterize``, the bit-exact
         replacement of the loader's per-record loop, loading_ipb.py:328-369) -- 0.5 instead of 25.8 MB per 720p frame
-        over the bus; only ``lq`` is then streamed in chunks."""
+        over the bus; only ``lq`` is then streamed in chunks.  A frame window's entry (``sideinfo.window_side``) is
+        rasterised by ``pnp_mv_rasterize_window``."""
         t = host_clip["lq"].shape[1]
         slot = self.turn
         self.turn ^= 1
@@ -402,7 +438,7 @@ class ClipStreamer:
                 from . import sideinfo
                 for c in range(n):
                     rec, meta, nbytes = sideinfo.upload_side(side[c], self.dev)
-                    side_dev.append((rec, meta))
+                    side_dev.append((rec, meta, side[c].get("tail")))
                     side_bytes += nbytes
                 side_ev = torch.cuda.Event()
                 side_ev.record(self.up)
@@ -468,11 +504,11 @@ class ClipStreamer:
             if self.raster_status is None:
                 self.raster_status = torch.zeros(1, dtype=torch.int32, device=self.dev)
             with torch.cuda.device(self.dev):
-                for c, (rec, meta) in enumerate(ticket["side_dev"]):
+                for c, (rec, meta, tail) in enumerate(ticket["side_dev"]):
                     rec.record_stream(main)          # allocated on the copy stream, read here
                     meta.record_stream(main)
                     sideinfo.rasterize_uploaded(rec, meta, t, dclip["mvs"][c], dclip["partitions"][c],
-                                                self.raster_work, self.raster_status)
+                                                self.raster_work, self.raster_status, tail)
             ticket["side_dev"] = []
         from .synthetic import generator_args
         # result buffers are owned here and recycled under events: a fresh torch.empty per clip that another stream

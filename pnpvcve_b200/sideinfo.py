@@ -36,16 +36,19 @@ def p_targets(slice_types):
     return tgt
 
 
-def _launch(rec, offs, is_b, tgt, t, h, w, work, mvs, par, status):
-    """pnp_mv_rasterize on the current stream of the tensors' device; ``work`` (3,T,H,W) int32 must be zeroed."""
+def _launch(rec, offs, is_b, tgt, t, h, w, work, mvs, par, status, tail=None):
+    """pnp_mv_rasterize on the current stream of the tensors' device; ``work`` (3,T,H,W) int32 must be zeroed.
+    ``tail`` (0 or 1) makes it pnp_mv_rasterize_window on a ``window_side`` table of T frames + ``tail`` tail frames."""
     lib = _lib.load()
     vp = ctypes.c_void_p
     stream = vp(torch.cuda.current_stream(mvs.device).cuda_stream)
-    _lib.check(lib.pnp_mv_rasterize(vp(rec.data_ptr() if rec.numel() else 0), vp(offs.data_ptr()),
-                                    vp(is_b.data_ptr()), vp(tgt.data_ptr()), t, rec.shape[0], h, w,
-                                    vp(work[0].data_ptr()), vp(work[1].data_ptr()), vp(work[2].data_ptr()),
-                                    vp(mvs.data_ptr()), vp(par.data_ptr()), vp(status.data_ptr()), stream),
-               "pnp_mv_rasterize")
+    head = (vp(rec.data_ptr() if rec.numel() else 0), vp(offs.data_ptr()), vp(is_b.data_ptr()), vp(tgt.data_ptr()), t)
+    rest = (rec.shape[0], h, w, vp(work[0].data_ptr()), vp(work[1].data_ptr()), vp(work[2].data_ptr()),
+            vp(mvs.data_ptr()), vp(par.data_ptr()), vp(status.data_ptr()), stream)
+    if tail is None:
+        _lib.check(lib.pnp_mv_rasterize(*head, *rest), "pnp_mv_rasterize")
+    else:
+        _lib.check(lib.pnp_mv_rasterize_window(*head, int(tail), *rest), "pnp_mv_rasterize_window")
 
 
 def raise_for_status(st):
@@ -94,9 +97,44 @@ def pack_side(records, frame_offsets, slice_types):
         raise ValueError("frame_offsets must have T+1 entries")
     meta = np.concatenate([offs, np.asarray([1 if s == "B" else 0 for s in slice_types], dtype=np.int32),
                            np.asarray(p_targets(slice_types), dtype=np.int32)])
+    return _pinned_side(rec, torch.as_tensor(meta), t=t)
+
+
+def _pinned_side(rec, meta, **kw):
     pin = torch.cuda.is_available()
-    meta = torch.as_tensor(meta)
-    return dict(records=rec.pin_memory() if pin else rec, meta=meta.pin_memory() if pin else meta, t=t)
+    return dict(records=rec.pin_memory() if pin else rec, meta=meta.pin_memory() if pin else meta, **kw)
+
+
+def window_side(side, a, b):
+    """The packed side information of frames [a, b) of a clip, from the clip's ``pack_side`` entry: rasterised by
+    ``pnp_mv_rasterize_window``, it gives exactly frames [a, b) of the whole clip's planes.
+
+    Records: those of frames [a, b), then -- as a tail frame -- the direction>0 rows of frame e, the first non-B frame
+    >= b, when their target (the previous non-B frame) lies inside the window: no other later frame writes into it.
+    ``meta`` is [frame_offsets (n+1) | is_b (n) | p_target (n)] of the n = (b - a) + tail table frames, window-relative;
+    a target before the window becomes -2 (the write lands outside it), -1 (frame 0 of the clip has no target) stays.
+    Returns the ``pack_side`` form plus ``tail`` (0 or 1)."""
+    t = side["t"]
+    if not 0 <= a < b <= t:
+        raise ValueError(f"window [{a}, {b}) is not inside a clip of {t} frames")
+    meta = side["meta"].tolist()
+    offs, is_b, tgt = meta[:t + 1], meta[t + 1:2 * t + 1], meta[2 * t + 1:]
+    rec = side["records"]
+    parts = [rec[offs[a]:offs[b]]]
+    rel = [v - a if v >= a else (-2 if v >= 0 else v) for v in tgt[a:b]]
+    w_offs = [o - offs[a] for o in offs[a:b + 1]]
+    w_is_b = list(is_b[a:b])
+    e = next((f for f in range(b, t) if not is_b[f]), None)
+    tail = int(e is not None and tgt[e] >= a)
+    if tail:
+        rows = rec[offs[e]:offs[e + 1]]
+        rows = rows[rows[:, 0] > 0]
+        parts.append(rows)
+        w_offs.append(w_offs[-1] + rows.shape[0])
+        w_is_b.append(0)
+        rel.append(tgt[e] - a)
+    return _pinned_side(torch.cat(parts, 0).contiguous(), torch.tensor(w_offs + w_is_b + rel, dtype=torch.int32),
+                        t=b - a, tail=tail)
 
 
 def mv_record_path(frame_path, dataset="reds"):
@@ -136,15 +174,17 @@ def upload_side(side, device):
     return rec, meta, rec.numel() * 4 + meta.numel() * 4
 
 
-def rasterize_uploaded(rec, meta, t, mvs, par, work, status):
+def rasterize_uploaded(rec, meta, t, mvs, par, work, status, tail=None):
     """Rasterise uploaded side information (``upload_side``) into ``mvs`` (T,4,H,W) / ``par`` (T,3,H,W) on the CURRENT
     stream without any host synchronisation; ``work`` (3,T,H,W) int32 is zeroed here, ``status`` accumulates the error
-    bits (check it with ``raise_for_status`` after a synchronisation)."""
+    bits (check it with ``raise_for_status`` after a synchronisation).  ``tail``: the entry is a frame window
+    (``window_side``) of T frames with that many (0 or 1) tail frames; None: a whole clip (``pack_side``)."""
     h, w = mvs.shape[-2], mvs.shape[-1]
-    if tuple(mvs.shape) != (t, 4, h, w) or tuple(par.shape) != (t, 3, h, w) or meta.numel() != 3 * t + 1:
+    n = t + (tail or 0)
+    if tuple(mvs.shape) != (t, 4, h, w) or tuple(par.shape) != (t, 3, h, w) or meta.numel() != 3 * n + 1:
         raise ValueError(f"side information of {t} frames does not match outputs {tuple(mvs.shape)} / {tuple(par.shape)}")
     work.zero_()
-    _launch(rec, meta[:t + 1], meta[t + 1:2 * t + 1], meta[2 * t + 1:], t, h, w, work, mvs, par, status)
+    _launch(rec, meta[:n + 1], meta[n + 1:2 * n + 1], meta[2 * n + 1:], t, h, w, work, mvs, par, status, tail)
 
 
 def synthetic_records(h, w, pattern, seed=0, messy=False):
