@@ -233,6 +233,26 @@ int pnp_unit_from_u8(const uint8_t* src, int64_t s_sf, int64_t s_sc, int64_t s_s
                      int64_t d_sc, int64_t d_sy, int F, int H, int W, void* stream);
 
 /*
+ * 8-bit frames -> PNG files, on the device.  The reference's test loop writes every output frame with
+ * mmcv.imwrite(tensor2img(frame)) (tools/test.py --save-path, forward_test(save_image=True)); OpenCV stores the BGR array
+ * as an RGB PNG, so PNG f holds exactly the uint8 frame f as 8-bit truecolour RGB (colour type 2, no interlace, no alpha;
+ * red = channel 0), at the size of the frame tensor.  The pixels are OpenCV's, the compressed bytes are not: filtered
+ * scanlines in segments of whole rows, LZ77 with fixed-Huffman blocks (or stored blocks where those are not larger),
+ * one IDAT chunk per segment.  A file depends on its frame's pixels and (H, W) only, not on F, batching or the stream.
+ *   frames : uint8 (F,3,H,W) view, unit x stride; sf/sc/sy = frame / channel / row strides in bytes
+ *   out    : PNG f is written at out + f * out_frame_stride (>= pnp_png_frame_bound(H, W) when F > 1), its length to
+ *            out_sizes[f] (device int64)
+ *   workspace : device memory of pnp_png_workspace_bytes(F, H, W) bytes, 16-byte aligned; no state is kept in it
+ * 1 <= F <= 65535, H >= 1, 1 <= W <= 21844.  pnp_png_frame_bound is the exact size of the largest file (every segment a
+ * stored block), chunk framing included; pnp_png_frame_bound / pnp_png_workspace_bytes return PNP_ERR_ARG for bad sizes.
+ * Additions: the ABI version and every other entry point are unchanged.
+ */
+int64_t pnp_png_frame_bound(int H, int W);
+int64_t pnp_png_workspace_bytes(int F, int H, int W);
+int pnp_png_encode(const uint8_t* frames, int64_t sf, int64_t sc, int64_t sy, int F, int H, int W, uint8_t* out,
+                   int64_t out_frame_stride, int64_t* out_sizes, void* workspace, int64_t workspace_bytes, void* stream);
+
+/*
  * K2/K3/K5 -- fused 3x3 convolution on tcgen05 tensor cores (implicit GEMM, TMA fed, TMEM
  * accumulators).  One call replaces one F.conv2d of the reference plus the elementwise work
  * around it:

@@ -21,7 +21,7 @@ EXPORTS = [
     "pnp_mv_warp", "pnp_mv_warp_dyn", "pnp_lr_im2col", "pnp_lr_im2col_dyn", "pnp_pack_conv3x3_rowstack",
     "pnp_pack_rows", "pnp_pack_aux", "pnp_pack_mix_blocks",
     "pnp_caa_heads", "pnp_mix_bias", "pnp_mv_rasterize", "pnp_conv3x3", "pnp_frame_quality", "pnp_frame_quality_u8",
-    "pnp_unit_from_u8", "pnp_mv_rasterize_window",
+    "pnp_unit_from_u8", "pnp_mv_rasterize_window", "pnp_png_frame_bound", "pnp_png_workspace_bytes", "pnp_png_encode",
 ]
 
 _c = ctypes
@@ -85,6 +85,9 @@ _PROTOS = {
     "pnp_frame_quality": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pnp_frame_quality_u8": (_i, [_vp, _i, _i64, _i64, _i64, _vp, _i, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pnp_unit_from_u8": (_i, [_vp, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _vp]),
+    "pnp_png_frame_bound": (_i64, [_i, _i]),
+    "pnp_png_workspace_bytes": (_i64, [_i, _i, _i]),
+    "pnp_png_encode": (_i, [_vp, _i64, _i64, _i64, _i, _i, _i, _vp, _i64, _vp, _vp, _i64, _vp]),
 }
 
 _lib = None

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpnpvcve.so")
-SOURCES = ["pnp_api.cu", "pnp_conv_rows.cu", "pnp_ops.cu", "pnp_raster.cu", "pnp_metrics.cu"]
+SOURCES = ["pnp_api.cu", "pnp_conv_rows.cu", "pnp_ops.cu", "pnp_raster.cu", "pnp_metrics.cu", "pnp_png.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-Xptxas", "-v"]
 

@@ -5,10 +5,14 @@ distributed_sampler.py:51-72) and gathers pickled results with two all_gathers
 (mmedit/apis/test.py:190-234).  Clips are independent, so here clip ``c`` goes to rank
 ``c mod world`` and the only communication is ONE fixed-shape all_gather of per-frame metrics.
 """
+import threading
 import weakref
+from concurrent.futures import ThreadPoolExecutor
 
 import torch
 import torch.distributed as dist
+
+from . import pngio
 
 N_METRICS = 2  # per frame: max-abs error vs. a reference frame (or 0), mean squared error
 
@@ -62,7 +66,7 @@ def gather_metrics(local, num_clips, rank, world, group=None):
 
 @torch.no_grad()
 def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=0, device=None, out_hosts=None,
-                  chunk=10, out_dtype=torch.float32):
+                  chunk=10, out_dtype=torch.float32, save_png=None):
     """Run this rank's share of ``clips``: a list of clip dicts as produced by pnpvcve_b200.synthetic, each holding
     n >= 1 equally shaped clips (n, T, ...); entries of other ranks may be None.
 
@@ -80,11 +84,24 @@ def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=
     and ``out_dtype=torch.uint8`` returns tensor2img's uint8 frames (mmedit/core/misc.py:9-74) of the fp32 result,
     stored by the last conv itself -- same (n,T,3,H,W) layout, a quarter of the bytes over the bus and in pinned
     memory.  ``out_hosts`` must then be uint8; ``gts`` / ``refs`` may be uint8 too.
+
+    ``save_png``: a callable (clip, frame) -> path that saves every frame as a PNG file, as the reference's
+    ``forward_test(save_image=True)`` does with ``mmcv.imwrite(tensor2img(...))``; clip is the row of the returned
+    metrics (``entry * n + j``).  mmedit's naming is one such callable:
+    ``lambda c, i: f"{save_path}/{folders[c]}/{i:08d}.png"``.  Needs ``out_dtype=torch.uint8``.  The files are encoded
+    on the device (``pngio``, pixel-identical to OpenCV's).  The frames of host entries are not downloaded -- their PNG
+    buffers are, written by host threads while later frames are computed -- and their ``outs`` are None;
+    device-resident entries return their frames as before.  The call returns after every file has been written and
+    raises the first OSError of a write.
     """
     from .synthetic import generator_args
     from . import metrics as _metrics
     if out_dtype not in (torch.float32, torch.uint8):
         raise ValueError(f"out_dtype must be torch.float32 or torch.uint8, got {out_dtype}")
+    if save_png is not None and out_dtype != torch.uint8:
+        raise ValueError("save_png needs out_dtype=torch.uint8 (PNG files hold tensor2img's uint8 frames)")
+    if save_png is not None and out_hosts is not None:
+        raise ValueError("save_png does not download the frames of host entries; leave out_hosts at None")
     if out_hosts is not None:
         bad = [c for c, o in enumerate(out_hosts) if o is not None and o.dtype != out_dtype]
         if bad:
@@ -113,12 +130,17 @@ def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=
         streamer = streamer_for(net, dev, chunk)
         ticket = streamer.upload(pinned[mine[0]])
         for i, c in enumerate(mine):
-            dst = out_hosts[c] if out_hosts is not None else \
-                torch.empty((n, t, 3, shape_of[-2] * up, shape_of[-1] * up), dtype=out_dtype).pin_memory()
-            out = streamer.run(ticket, dst)
+            oshape = (n, t, 3, shape_of[-2] * up, shape_of[-1] * up)
+            if save_png is not None:        # the frames stay on the device (a meta tensor carries shape and dtype)
+                dst = torch.empty(oshape, dtype=out_dtype, device="meta")
+                png = lambda j, k, c=c: save_png(c * n + j, k)        # noqa: E731
+            else:
+                dst = out_hosts[c] if out_hosts is not None else torch.empty(oshape, dtype=out_dtype).pin_memory()
+                png = None
+            out = streamer.run(ticket, dst) if png is None else streamer.run(ticket, dst, png=png)
             ticket = streamer.upload(pinned[mine[i + 1]]) if i + 1 < len(mine) else None   # overlaps clip c's kernels
             measure(c, out)                 # on the device copy, before its buffer is recycled two entries later
-            outs.append(dst)
+            outs.append(None if save_png is not None else dst)
         streamer.finish(check=True)
     else:
         for c in mine:
@@ -132,6 +154,8 @@ def enhance_clips(net, clips, rank=0, world=1, refs=None, gts=None, crop_border=
                 out = net(*generator_args(clips[c]))
             outs.append(out)
             measure(c, out)
+            if save_png is not None:
+                pngio.save_frames(out, lambda j, k, c=c: save_png(c * n + j, k))
     nm = N_METRICS + (2 if gts is not None else 0)
     local = torch.cat(mets, 0) if mets else torch.empty((0, t, nm), device=dev)
     per_entry = gather_metrics(local.view(len(mine), n * t, nm) if mets else local.view(0, n * t, nm),
@@ -191,7 +215,7 @@ def _pinned(v):
 
 @torch.no_grad()
 def enhance_windows(net, clips, window, rank=0, world=1, overlap=0, refs=None, gather_output=False, group=None,
-                    device=None, chunk=10, gts=None, crop_border=0, out_dtype=torch.float32):
+                    device=None, chunk=10, gts=None, crop_border=0, out_dtype=torch.float32, save_png=None):
     """Frame-window sharding (north_star: "sharding independent clips or frame windows per GPU"): the windows of
     ``clips`` (equally shaped (1,T,...) clip dicts) are dealt to the ranks round robin and enhanced independently.
     HOST-resident clips stream their windows through the cached ``ClipStreamer`` of (net, device, chunk) on ``device``
@@ -206,6 +230,11 @@ def enhance_windows(net, clips, window, rank=0, world=1, overlap=0, refs=None, g
     last conv (as in ``enhance_clips``).  ``gts`` (per clip (1,T,3,H,W), fp32 or uint8) adds PSNR / SSIM
     (``metrics.frame_quality`` with ``crop_border``) to every frame's metric vector: [max-abs, mse, PSNR, SSIM].
 
+    ``save_png``: a callable (clip, frame) -> path, frame counted in the whole clip, that saves the core frames of every
+    window (never its overlap frames) as PNG files encoded on the device, as in ``enhance_clips`` -- so each frame of a
+    clip is written exactly once, by the rank that owns it.  Needs ``out_dtype=torch.uint8`` and excludes
+    ``gather_output``; the frames of host clips are then not downloaded.
+
     Returns (outs, metrics): outs = {(clip, a, b): (1, b-a, 3, H, W) frames} of this rank's windows (device tensors)
     -- or, with ``gather_output``, the complete (num_clips, T, 3, H, W) result on every rank (one fixed-shape all_gather
     of frames over NVLink, in ``out_dtype``) --, metrics = (num_clips, T, M) of ALL frames on every rank (one
@@ -214,6 +243,10 @@ def enhance_windows(net, clips, window, rank=0, world=1, overlap=0, refs=None, g
     from . import metrics as _metrics
     if out_dtype not in (torch.float32, torch.uint8):
         raise ValueError(f"out_dtype must be torch.float32 or torch.uint8, got {out_dtype}")
+    if save_png is not None and out_dtype != torch.uint8:
+        raise ValueError("save_png needs out_dtype=torch.uint8 (PNG files hold tensor2img's uint8 frames)")
+    if save_png is not None and gather_output:
+        raise ValueError("save_png writes each rank's own windows; it cannot be combined with gather_output")
     num_clips = len(clips)
     t = clips[0]["lq"].shape[1]
     # host-resident clips are streamed when `net` is the generator (anything else -- a stand-in callable in the CPU tests
@@ -240,9 +273,13 @@ def enhance_windows(net, clips, window, rank=0, world=1, overlap=0, refs=None, g
         if host:
             hwin, lo, hi = wins[i]
             shape = (1, hwin["lq"].shape[1], 3, hwin["lq"].shape[-2] * up, hwin["lq"].shape[-1] * up)
-            if shape not in dsts:     # one download target per window shape, written in stream order
+            png = None
+            if save_png is not None:  # core frames only, numbered in the whole clip; no frame download
+                dsts.setdefault(shape, torch.empty(shape, dtype=out_dtype, device="meta"))
+                png = lambda j, k, c=c, lo=lo, hi=hi, a0=a - lo: save_png(c, a0 + k) if lo <= k < hi else None  # noqa
+            elif shape not in dsts:   # one download target per window shape, written in stream order
                 dsts[shape] = _pinned(torch.empty(shape, dtype=out_dtype))
-            full = streamer.run(ticket, dsts[shape])
+            full = streamer.run(ticket, dsts[shape]) if png is None else streamer.run(ticket, dsts[shape], png=png)
             ticket = streamer.upload(wins[i + 1][0]) if i + 1 < len(mine) else None
             out = full[:, lo:hi].clone()            # (the streamer recycles its device buffer two windows later)
         else:
@@ -255,6 +292,8 @@ def enhance_windows(net, clips, window, rank=0, world=1, overlap=0, refs=None, g
                 out = net.forward_streamed(*args, out=buf)[:, lo:hi]
             else:
                 out = net(*args)[:, lo:hi]
+            if save_png is not None:
+                pngio.save_frames(out, lambda j, k, c=c, a=a: save_png(c, a + k))
         outs[(c, a, b)] = out
         m = frame_metrics(out, None if refs is None else refs[c][:, a:b].to(dev))[0]
         if gts is not None:
@@ -342,7 +381,18 @@ class ClipStreamer:
     chunk in and the last chunk out.  A call takes a batch of n >= 1 clips (n, T, ...): every copy is issued per clip
     so that it is one contiguous DMA transfer (a strided (n, chunk) slice of a pinned tensor would be staged through a
     pageable bounce buffer by the framework and stall the host).
+
+    PNG files (``run(..., png=...)``): at the end of each chunk its frames are encoded on the kernels' stream
+    (``pngio.encode``; on a side stream the encoder would share the SMs with the persistent conv kernels and slow them),
+    the files go down on the download stream into pinned buffers (the whole frame bound per frame), and a small pool of
+    host threads writes them once that copy has completed.  The kernels' stream never waits on the host; at most
+    ``PNG_IN_FLIGHT`` chunks wait for their writes, and ``finish`` joins the writers.
     """
+
+    PNG_WRITERS = 4
+    #: chunks whose pinned PNG buffers may wait for their writes; beyond that the host (never the kernels' stream) waits
+    #: for the oldest write, so that a slow disk cannot make locked host memory grow with the length of a call
+    PNG_IN_FLIGHT = 8
 
     BIG = ("lq", "mvs", "partitions")
     SMALL = ("QPs", "slices", "base_QPs")
@@ -361,6 +411,12 @@ class ClipStreamer:
         self.turn = 0
         self.h2d_bytes = self.d2h_bytes = 0
         self.raster_work = self.raster_status = None     # compact side information: rasteriser workspace / error bits
+        self.pngs = [None, None]           # per slot: (device PNG buffer, sizes, event "its last download has finished")
+        self._png_host = {}                # (frames, bound) -> free pinned (buffer, sizes) pairs
+        self._png_lock = threading.Lock()
+        self._writers = None               # ThreadPoolExecutor, created on first use
+        self._png_jobs = []
+        self._png_error = None
         #: diagnostics (tools/e2e_probe.py): skip the big H2D / D2H copies to see what each direction costs
         self.copy_in = self.copy_out = True
 
@@ -456,9 +512,11 @@ class ClipStreamer:
                     cond=(host_clip["slices"], host_clip["base_QPs"], host_clip["QPs"]))
 
     @torch.no_grad()
-    def run(self, ticket, out_host):
+    def run(self, ticket, out_host, png=None):
         """Enqueue the kernels of an uploaded clip and the chunked download of its frames into ``out_host`` (fp32, or
-        uint8: the last conv then stores tensor2img's uint8 frames)."""
+        uint8: the last conv then stores tensor2img's uint8 frames).  An ``out_host`` on the meta device only gives the
+        shape and dtype: the frames are then not downloaded.  ``png``: a callable (clip of the batch, frame) -> path or
+        None; the uint8 frames with a path are saved as PNG files (see the class docstring)."""
         main = torch.cuda.current_stream(self.dev)
         t, dclip, events = ticket["t"], ticket["dclip"], ticket["events"]
         chunks = self._chunks(t)
@@ -482,14 +540,19 @@ class ClipStreamer:
             if c not in waited:
                 arrive(c)
 
+        download = self.copy_out and out_host.device.type != "meta"
+        png_bytes = [0]
+
         def frame_done(i, out):
             a, b = owner[i]
             if i == b - 1:
+                if png is not None:
+                    png_bytes[0] += self._png_chunk(out, a, b, png, main, slot)
                 ev = torch.cuda.Event()
                 ev.record(main)
                 with torch.cuda.stream(self.down):
                     self.down.wait_event(ev)
-                    for c in range(out.shape[0]) if self.copy_out else ():
+                    for c in range(out.shape[0]) if download else ():
                         out_host[c, a:b].copy_(out[c, a:b], non_blocking=True)
 
         arrive(chunks[-1])                           # small tensors + the first chunk the kernels need
@@ -514,6 +577,16 @@ class ClipStreamer:
         # result buffers are owned here and recycled under events: a fresh torch.empty per clip that another stream
         # still reads (record_stream) keeps the caching allocator from reusing the block and ends in cudaMalloc stalls
         slot = ticket["slot"]
+        if png is not None:
+            if out_host.dtype != torch.uint8:
+                raise ValueError("PNG files are written from uint8 frames")
+            bound = pngio.frame_bound(out_host.shape[-2], out_host.shape[-1])
+            pshape = tuple(out_host.shape[:2]) + (bound,)
+            if self.pngs[slot] is not None and self.pngs[slot][2] is not None:
+                main.wait_event(self.pngs[slot][2])  # (also before a buffer of another shape replaces it)
+            if self.pngs[slot] is None or tuple(self.pngs[slot][0].shape) != pshape:
+                self.pngs[slot] = (torch.empty(pshape, dtype=torch.uint8, device=self.dev),
+                                   torch.empty(pshape[:2], dtype=torch.int64, device=self.dev), None)
         if self.outs[slot] is not None and tuple(self.outs[slot][0].shape) == tuple(out_host.shape) and \
                 self.outs[slot][0].dtype == out_host.dtype:
             obuf, free_ev = self.outs[slot]
@@ -525,16 +598,74 @@ class ClipStreamer:
         free_ev = torch.cuda.Event()
         free_ev.record(self.down)                    # behind the last chunk's download
         self.outs[slot] = (obuf, free_ev)
+        if png is not None:
+            self.pngs[slot] = self.pngs[slot][:2] + (free_ev,)
         done = torch.cuda.Event()
         done.record(main)
         self.slots[ticket["slot"]] = (self.slots[ticket["slot"]][0], dclip, done)
-        self.d2h_bytes = out.numel() * out.element_size()
+        self.d2h_bytes = (out.numel() * out.element_size() if download else 0) + png_bytes[0]
         return out
+
+    def _png_chunk(self, out, a, b, png, main, slot):
+        """Encode frames [a, b) of every clip of ``out`` that have a path (on the kernels' stream), enqueue their download
+        into pinned buffers and hand the writes to the writer threads.  Returns the bytes copied."""
+        n = out.shape[0]
+        paths = [[png(c, i) for i in range(a, b)] for c in range(n)]
+        have = [k for k in range(b - a) if any(p[k] is not None for p in paths)]
+        if not have:
+            return 0
+        lo, hi = a + have[0], a + have[-1] + 1
+        pbuf, psizes = self.pngs[slot][:2]
+        with torch.cuda.stream(main), torch.cuda.device(self.dev):
+            for c in range(n):
+                pngio.encode(out[c, lo:hi], out=pbuf[c, lo:hi], sizes=psizes[c, lo:hi])
+        ev = torch.cuda.Event()
+        ev.record(main)
+        key = (n * (hi - lo), pbuf.shape[-1])
+        while len(self._png_jobs) >= self.PNG_IN_FLIGHT:
+            self._png_jobs.pop(0).result()
+        with self._png_lock:
+            free = self._png_host.setdefault(key, [])
+            hbuf, hsizes = free.pop() if free else (torch.empty(key, dtype=torch.uint8, pin_memory=True),
+                                                     torch.empty(key[0], dtype=torch.int64, pin_memory=True))
+        with torch.cuda.stream(self.down):
+            self.down.wait_event(ev)
+            for c in range(n):
+                k = slice(c * (hi - lo), (c + 1) * (hi - lo))
+                hbuf[k].copy_(pbuf[c, lo:hi], non_blocking=True)
+                hsizes[k].copy_(psizes[c, lo:hi], non_blocking=True)
+            copied = torch.cuda.Event()
+            copied.record(self.down)
+        if self._writers is None:
+            self._writers = ThreadPoolExecutor(max_workers=self.PNG_WRITERS, thread_name_prefix="png-writer")
+        flat = [p[i - a] for p in paths for i in range(lo, hi)]
+        self._png_jobs.append(self._writers.submit(self._png_write, copied, hbuf, hsizes, flat, key))
+        return hbuf.numel() + hsizes.numel() * hsizes.element_size()
+
+    def _png_write(self, copied, hbuf, hsizes, paths, key):
+        """writer thread: wait for the download, write the files, return the pinned buffers to the pool"""
+        try:
+            copied.synchronize()
+            if self._png_error is None:
+                pngio.write(hbuf, hsizes, paths)
+        except OSError as e:
+            with self._png_lock:
+                if self._png_error is None:
+                    self._png_error = e
+        finally:
+            with self._png_lock:
+                self._png_host[key].append((hbuf, hsizes))
 
     def finish(self, check=False):
         """Order the caller's stream behind the last download.  ``check``: synchronise and raise what the reference's
         loader raises for malformed side information (KeyError / ValueError, see sideinfo.raise_for_status)."""
         torch.cuda.current_stream(self.dev).wait_stream(self.down)
+        jobs, self._png_jobs = self._png_jobs, []
+        for j in jobs:
+            j.result()
+        if check and self._png_error is not None:
+            err, self._png_error = self._png_error, None
+            raise err
         if check and self.raster_status is not None:
             from . import sideinfo
             st = int(self.raster_status.item())
