@@ -475,14 +475,20 @@ class ClipStreamer:
             shapes["lq_u8"] = shapes["lq"]
             shapes["lq"] = (shapes["lq"][0], torch.float32)
         key = tuple((k, sh, dt) for k, (sh, dt) in sorted(shapes.items()))
-        if self.slots[slot] is None or self.slots[slot][0] != key:
+        fresh = self.slots[slot] is None or self.slots[slot][0] != key
+        if fresh:
             self.slots[slot] = (key, {k: torch.empty(sh, dtype=dt, device=self.dev) for k, (sh, dt) in shapes.items()},
                                 None)
         dclip = self.slots[slot][1]
         busy = self.slots[slot][2]         # kernels of the clip that last used these buffers
         events = {}
         side_bytes, side_dev, side_ev = 0, [], None
+        main = torch.cuda.current_stream(self.dev)
         with torch.cuda.stream(self.up):
+            if fresh:
+                # new buffers come from the caller's stream's pool: a block freed there may still be written by work
+                # enqueued on that stream (the previous clip's temporaries), so the copies into it wait for that work
+                self.up.wait_stream(main)
             if busy is not None:
                 self.up.wait_event(busy)
             for k in self.SMALL:
@@ -587,10 +593,11 @@ class ClipStreamer:
             if self.pngs[slot] is None or tuple(self.pngs[slot][0].shape) != pshape:
                 self.pngs[slot] = (torch.empty(pshape, dtype=torch.uint8, device=self.dev),
                                    torch.empty(pshape[:2], dtype=torch.int64, device=self.dev), None)
+        if self.outs[slot] is not None:
+            main.wait_event(self.outs[slot][1])      # (also before a buffer of another shape replaces it)
         if self.outs[slot] is not None and tuple(self.outs[slot][0].shape) == tuple(out_host.shape) and \
                 self.outs[slot][0].dtype == out_host.dtype:
-            obuf, free_ev = self.outs[slot]
-            main.wait_event(free_ev)
+            obuf = self.outs[slot][0]
         else:
             obuf = torch.empty(out_host.shape, dtype=out_host.dtype, device=self.dev)
         out = self.net.forward_streamed(*generator_args(dclip), cond_host=ticket["cond"], frame_ready=frame_ready,

@@ -58,20 +58,25 @@ def test_generator_matches_reference_golden(dev, name):
     print(f"{name}: max-abs vs reference golden {err:.2e}")
 
 
-@pytest.mark.parametrize("name", ["c1_128x128_t7", "n2_64x96_t6_ipb", "edge_68x132_t3"])
-def test_generator_in_pair_form_matches_reference_golden(dev, name):
-    """The whole generator with every eligible conv launch in the CTA-pair (cta_group::2) form, phantom columns
-    included: same reference goldens, and bit-identical to the default form."""
+@pytest.mark.parametrize("mode", [1, 2])
+@pytest.mark.parametrize("name", CASES)
+def test_generator_in_pair_form_matches_reference_golden(dev, name, mode):
+    """The whole generator with every eligible conv launch in the CTA-pair (cta_group::2) form (mode 2: phantom
+    columns included), for every golden case with its vsr / sparse_val flags: same reference goldens, and bit-identical
+    to the default form.  Catches a pair-form defect on an optional path: the strided PixelShufflePack stores of the vsr
+    tail, the sparse partition blend, all-B / mirrored / one-frame schedules."""
     from pnpvcve_b200 import _lib
     lib = _lib.load()
     sd, clip, gold = build_case(name)
-    ref = run(build(sd, dev), clip, dev)
-    prev = lib.pnp_set_pair_mode(2)
+    case = golden_cases()[name]
+    flags = dict(vsr=bool(case.get("vsr")), sparse_val=bool(case.get("sparse_val")))
+    ref = run(build(sd, dev, **flags), clip, dev)
+    prev = lib.pnp_set_pair_mode(mode)
     try:
-        out = run(build(sd, dev), clip, dev)
+        out = run(build(sd, dev, **flags), clip, dev)
     finally:
         lib.pnp_set_pair_mode(prev)
-    check_against_golden(out, gold, tol=TOL, lq=clip["lq"], vsr=False)
+    check_against_golden(out, gold, tol=TOL, lq=clip["lq"], vsr=flags["vsr"])
     assert torch.equal(out, ref)
 
 
@@ -202,6 +207,51 @@ def test_clip_streamer_equals_plain_forward(dev):
         assert torch.equal(o, r)
     assert st.h2d_bytes == sum(v.numel() * v.element_size() for v in hosts[0].values())
     assert st.d2h_bytes == refs[0].numel() * 4
+
+
+def test_clip_streamer_orders_fresh_buffers_behind_pending_work(dev):
+    """ClipStreamer takes new device buffers from the caller's stream's pool whenever a clip shape changes (frame
+    windows of different lengths), but fills its input buffers on the upload stream and empties its result buffers on
+    the download stream.  A block freed by work still queued on one stream must not be written through another before
+    that work is done: the upload into fresh input buffers waits for the caller's stream, and a result buffer of another
+    shape replaces the old one only behind the old one's download.  Without that order the next clip's inputs can land
+    in a block that a queued kernel still writes (seen as frame-window metrics that differ between identical calls).
+    A long sleep on one stream makes the order observable."""
+    from pnpvcve_b200 import driver
+    sd = weights.random_state_dict(9, num_blocks=2)
+    net = build(sd, dev, num_blocks=2)
+    clips = [synthetic.make_clip(64, 96, t, seed=620 + t) for t in (4, 4, 2)]
+    refs = [run(net, c, dev).cpu() for c in clips]
+    hosts = [{k: v.pin_memory() for k, v in c.items()} for c in clips]
+    outs = [torch.empty_like(r).pin_memory() for r in refs]
+    sleep = 10 ** 9                                  # cycles: ~0.5 s, far longer than these clips' launches
+    st = driver.ClipStreamer(net, dev, chunk=4)
+    main = torch.cuda.current_stream(dev)
+    torch.cuda.synchronize()
+    torch.cuda._sleep(sleep)
+    busy = torch.cuda.Event()
+    busy.record(main)
+    ticket = st.upload(hosts[0])                     # fresh input buffers
+    for ev in ticket["events"].values():
+        ev.synchronize()
+    assert busy.query(), "the upload into fresh buffers overtook work queued on the caller's stream"
+    with torch.cuda.stream(st.down):                 # clip 0's downloads queue up behind a sleep
+        torch.cuda._sleep(sleep)
+        slow = torch.cuda.Event()
+        slow.record(st.down)
+    st.run(ticket, outs[0])                          # slot 0
+    ticket = st.upload(hosts[1])
+    st.run(ticket, outs[1])                          # slot 1
+    ticket = st.upload(hosts[2])
+    st.run(ticket, outs[2])                          # slot 0 again, T=2: a new result buffer replaces clip 0's
+    done = torch.cuda.Event()
+    done.record(main)
+    done.synchronize()
+    assert slow.query(), "a result buffer was replaced before its download had finished"
+    st.finish()
+    torch.cuda.synchronize()
+    for o, r in zip(outs, refs):
+        assert torch.equal(o, r)
 
 
 def test_frame_windows_match_oracle_on_the_same_windows(dev):
